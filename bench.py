@@ -14,6 +14,10 @@ fwd/bwd/AdamW + loss.item() per step).  `roofline` = dominant kernel of the step
 (CUDA events on the launching stream, separate instrumented pass over the same steps), algorithmic
 bytes or flops per launch / average duration, against MEASURED_PEAKS.json.  `cpu_baseline` = the
 oracle on the box's host cores on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the timed device-resident training step computed in its last step
+(its loss and the parameters its AdamW update left in the model, float32) as DIR/<name>.npy.  Every
+input is seeded, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -123,6 +127,16 @@ class ClockSampler:
             return {"sm_mhz": float(np.median(self.samples)) if self.samples else None, "sm_max_mhz": float(self.max),
                     "reasons": sorted(self.reasons), "samples": len(self.samples)}
         return {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "error": getattr(self, "err", "nvml unavailable")}
+
+
+def dump_outputs(out_dir, loss, model):
+    """The last timed training step's loss and the parameters it left in ``model``, one float32 ``.npy`` per array
+    (``loss.npy``, ``param.<name>.npy``): about 0.6 MB for the benchmarked model."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().reshape(1)}
+    arrays.update({f"param.{k}": p.detach() for k, p in model.named_parameters()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def timed_region(step_fn, steps, dist_on, device):
@@ -614,7 +628,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the tet-batch, config-4 aggregation and config-5 blocks")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels one by one instead of replaying CUDA graphs (both arms)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed training step's loss and parameters to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -704,7 +723,7 @@ def main():
         from deep_fem_uav_wing.gnn.graphed import GraphedTrainStep
 
         rstep = GraphedTrainStep(model, crit, opt, ddp=ddp)
-        replays = [rstep.capture_resident(b.x, g_, b.y, b.loss_mask)[0] for b, g_ in zip(resident, graphs)]
+        replays, rlosses = zip(*[rstep.capture_resident(b.x, g_, b.y, b.loss_mask) for b, g_ in zip(resident, graphs)])
         for i in range(min(3, n_batches)):
             replays[i]()
     sampler = ClockSampler(local_rank)
@@ -712,10 +731,20 @@ def main():
     k0 = ops.LAUNCH_COUNTER["kernels"]
     if replays is not None:
         ms_total = timed_region(lambda i: replays[(warmup + i) % n_batches](), steps, dist_on, device)
+        last_loss = rlosses[(warmup + steps - 1) % n_batches]
     else:
-        ms_total = timed_region(lambda i: train_step(resident[(warmup + i) % n_batches], graph=graphs[(warmup + i) % n_batches]), steps, dist_on, device)
+        eager_loss = [None]
+
+        def eager_step(i):
+            j = (warmup + i) % n_batches
+            eager_loss[0] = train_step(resident[j], return_loss=True, graph=graphs[j])
+
+        ms_total = timed_region(eager_step, steps, dist_on, device)
+        last_loss = eager_loss[0]
     launches = ops.LAUNCH_COUNTER["kernels"] - k0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss, model)  # before the later arms step the model further
     value = BATCH * steps * world / (ms_total * 1e-3)
 
     # ---- inference arm (BASELINE metric: "train/infer"): eval-mode forward over the same resident batches ----

@@ -95,12 +95,13 @@ def model_case(ref_model, name, mesh, hidden, layers, seed):
                              metrics["masked_nodes"]["max_error"], metrics["masked_nodes"]["count"]], dtype=np.float64),
     }
     rec.update(sd_to_np(model.state_dict(), "sd/"))
-    rec.update({f"grad/{k}": p.grad.detach().numpy() for k, p in model.named_parameters()})
+    grads = {f"grad/{k}": p.grad.detach().numpy() for k, p in model.named_parameters()}
     # eval-mode forward with the constructor-default dropout (must equal dropout-free forward)
     model.eval()
     with torch.no_grad():
         rec["out_eval"] = model(x, ei).numpy()
     np.savez_compressed(HERE / f"{name}.npz", **rec)
+    np.savez_compressed(HERE / f"{name}.grads.npz", **grads)  # apart, so that every file stays under 1 MB
     print(f"{name}: N={x.shape[0]} E={ei.shape[1]} loss={loss.item():.6f}")
 
 
