@@ -116,6 +116,12 @@ __host__ __device__ __forceinline__ uint32_t dropout_threshold(float p) {
     return static_cast<uint32_t>(t);
 }
 
+// The canonical CSR build of dfw_csr_build (dfw_csr.cu), shared with the vertex-normal build (dfw_screen.cu).  `gate`
+// (nullable, device) skips every kernel when *gate == 0.  ws: dfw_csr_ws_bytes(E, N).
+int csr_build_impl(const int64_t* edge_index, int64_t E, int64_t N, int by_src, int32_t* rowptr, int32_t* col,
+                   int32_t* perm, float* inv_deg, int32_t* status, void* ws, size_t ws_bytes, dfw_stream_t stream,
+                   const int32_t* gate);
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

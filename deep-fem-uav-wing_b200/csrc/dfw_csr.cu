@@ -274,7 +274,7 @@ extern "C" size_t dfw_csr_ws_bytes(int64_t E, int64_t N) {
 }
 
 namespace dfw {
-static int csr_build_impl(const int64_t* edge_index, int64_t E, int64_t N, int by_src, int32_t* rowptr, int32_t* col,
+int csr_build_impl(const int64_t* edge_index, int64_t E, int64_t N, int by_src, int32_t* rowptr, int32_t* col,
                           int32_t* perm, float* inv_deg, int32_t* status, void* ws, size_t ws_bytes, dfw_stream_t stream,
                           const int32_t* gate = nullptr);
 }
@@ -286,7 +286,7 @@ extern "C" int dfw_csr_build(const int64_t* edge_index, int64_t E, int64_t N, in
 }
 
 namespace dfw {
-static int csr_build_impl(const int64_t* edge_index, int64_t E, int64_t N, int by_src, int32_t* rowptr, int32_t* col,
+int csr_build_impl(const int64_t* edge_index, int64_t E, int64_t N, int by_src, int32_t* rowptr, int32_t* col,
                           int32_t* perm, float* inv_deg, int32_t* status, void* ws, size_t ws_bytes, dfw_stream_t stream,
                           const int32_t* gate) {
     DFW_REQUIRE(E >= 0 && N >= 0, "dfw_csr_build: negative size (E=%lld, N=%lld)", (long long)E, (long long)N);

@@ -7,7 +7,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import c_float, c_int, c_int64, c_size_t, c_uint64, c_void_p
+from ctypes import c_double, c_float, c_int, c_int64, c_size_t, c_uint64, c_void_p
 
 _PKG_ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), "..", ".."))
 LIB_PATH = os.environ.get("DFW_B200_LIB", os.path.join(_PKG_ROOT, "lib", "libdfw_b200.so"))
@@ -83,6 +83,11 @@ SIGNATURES = {
     "dfw_stress_metrics_ws_bytes": (c_size_t, [c_int64, c_int64]),
     "dfw_stress_metrics": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_size_t,
                                    c_void_p]),
+    "dfw_vertex_normals_ws_bytes": (c_size_t, [c_int64, c_int64]),
+    "dfw_vertex_normals": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dfw_case_stress_summary_ws_bytes": (c_size_t, [c_int64, c_int64]),
+    "dfw_case_stress_summary": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_double, c_double, c_int,
+                                        c_void_p, c_void_p, c_size_t, c_void_p]),
     "dfw_cast": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_void_p]),
 }
 

@@ -74,6 +74,43 @@ def load_packed_case(path) -> dict[str, Any]:
     return raw
 
 
+GEOMETRY_VERSION = 1
+
+
+def pack_geometry_case(out_path, case_id, node_id, pos, faces, params) -> Path:
+    """Write the pre-FEM content of a case - surface node ids and positions, faces as node ids, the four wing parameters
+    (a dict with ``span_m, chord_m, sweep_deg, thickness_ratio``) - as one uncompressed ``.npz``: what design screening
+    (``gnn/screening.py``) needs of a design that has not been through FEM.  Arrays are stored with their dtypes as given,
+    so :func:`load_geometry_case` returns them bit for bit.  Written atomically like :func:`pack_case`."""
+    node_id, pos, faces = np.asarray(node_id), np.asarray(pos), np.asarray(faces)
+    if pos.ndim != 2 or pos.shape[1] != 3 or node_id.shape != (pos.shape[0],):
+        raise ValueError(f"pos must be [N, 3] and node_id [N], got {pos.shape} and {node_id.shape}")
+    if faces.size % 3 or not np.issubdtype(faces.dtype, np.integer) or not np.issubdtype(node_id.dtype, np.integer):
+        raise ValueError("faces must be an integer [F, 3] array of node ids and node_id an integer array")
+    out_path = Path(out_path)
+    out_path.parent.mkdir(parents=True, exist_ok=True)
+    tmp = out_path.with_name(out_path.name + f".tmp{os.getpid()}")
+    with open(tmp, "wb") as f:
+        np.savez(f, geometry_version=np.int64(GEOMETRY_VERSION), case_id=np.array(str(case_id)), node_id=node_id, pos=pos,
+                 faces=faces.reshape(-1, 3), params=np.array([float(params[k]) for k in _PARAM_KEYS], dtype=np.float64))
+    os.replace(tmp, out_path)
+    return out_path
+
+
+def load_geometry_case(path) -> dict[str, Any]:
+    """Inverse of :func:`pack_geometry_case`: ``{case_id, node_id, pos, faces, params}``, the case dict
+    ``DesignScreener.screen`` takes."""
+    z = np.load(path, allow_pickle=False)
+    if "geometry_version" not in z.files:
+        raise ValueError(f"{path}: not a geometry case (no geometry_version field)")
+    version = int(z["geometry_version"])
+    if version != GEOMETRY_VERSION:
+        raise ValueError(f"{path}: geometry case version {version}, this build reads version {GEOMETRY_VERSION}")
+    p = z["params"]
+    return {"case_id": str(z["case_id"]), "node_id": z["node_id"], "pos": z["pos"], "faces": z["faces"],
+            "params": {k: float(p[i]) for i, k in enumerate(_PARAM_KEYS)}}
+
+
 def packed_path(root, case_id: str) -> Path:
     return Path(root) / "data" / "packed" / f"{case_id}.npz"
 

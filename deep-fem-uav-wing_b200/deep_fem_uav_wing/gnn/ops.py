@@ -766,6 +766,68 @@ def stress_metrics(pred, target, mask=None, log_scale=True) -> torch.Tensor:
     return result
 
 
+def vertex_normals(pos: torch.Tensor, faces: torch.Tensor):
+    """``dfw_vertex_normals``: area-weighted vertex normals fp32 [N,3] of a triangulated surface (reference ``fem.py:390-424``)
+    and an int32 [1] device count of the faces skipped for an index outside [0, N).  ``faces`` int64 [F,3] of 0-based rows.
+    Deterministic (ascending incidence order, no float atomics) and without host synchronisation."""
+    _require_cuda(pos, "pos")
+    _require_cuda(faces, "faces")
+    if faces.dtype != torch.int64:
+        raise TypeError(f"faces must be int64, got {faces.dtype}")
+    pos = pos.to(torch.float32).contiguous()
+    f = faces.reshape(-1, 3).contiguous()
+    N, F, dev = int(pos.shape[0]), int(f.shape[0]), pos.device
+    if 3 * F >= 2**31 - 1 or N >= 2**31 - 1:
+        raise ValueError("dfw_vertex_normals uses int32 incidence lists: 3F and N must be < 2^31")
+    normal = torch.empty(N, 3, dtype=torch.float32, device=dev)
+    status = torch.empty(1, dtype=torch.int32, device=dev)
+    ws_bytes = lib.dfw_vertex_normals_ws_bytes(F, N)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev), _prof("vertex_normals", 24 * F + 24 * N):
+        check(lib.dfw_vertex_normals(pos.data_ptr(), N, f.data_ptr(), F, normal.data_ptr(), status.data_ptr(), ws.data_ptr(), ws_bytes,
+                                     _stream(pos)))
+    LAUNCH_COUNTER["kernels"] += 9 if F > 0 else 4
+    return normal, status
+
+
+def case_stress_summary(pred, pos, case_ptr, mask=None, root_band: float = 0.05, allowable_pa: float | None = None,
+                        log_scale: bool = True) -> torch.Tensor:
+    """``dfw_case_stress_summary``: float64 [B,8] on the device, one record per case of ``case_ptr`` (int64 [B+1], device):
+    [rows, screened rows, max stress, its row within the case (-1: none), mean stress, max stress over all rows,
+    screened rows above ``allowable_pa``, non-finite stresses].  Screened rows are ``mask`` (uint8/bool [N]) or, without
+    it, ``pos_y > root_band * (max_y - min_y)`` of the case.  ``pred`` [N] or [N,1], fp32 or bf16, ``log1p(stress)`` when
+    ``log_scale``.  Deterministic and independent of how cases are batched; no host synchronisation."""
+    _require_cuda(pred, "pred")
+    p = pred.detach().contiguous()
+    N = int(p.shape[0]) if p.dim() > 0 else 1
+    if p.numel() != N:
+        raise ValueError(f"pred must be [N] or [N,1], got {tuple(pred.shape)}")
+    pos = pos.to(torch.float32).contiguous()
+    if tuple(pos.shape) != (N, 3):
+        raise ValueError(f"pos must be [{N}, 3], got {tuple(pos.shape)}")
+    if case_ptr.dtype != torch.int64 or case_ptr.device != p.device:
+        raise TypeError("case_ptr must be an int64 tensor on the device of pred")
+    cp = case_ptr.contiguous()
+    B = int(cp.numel()) - 1
+    if B < 0:
+        raise ValueError("case_ptr needs at least one entry")
+    m = None
+    if mask is not None:
+        m = mask.detach().reshape(-1).contiguous()
+        m = m.view(torch.uint8) if m.dtype == torch.bool else m.to(torch.uint8)
+        if m.numel() != N:
+            raise ValueError(f"mask has {m.numel()} entries for {N} rows")
+    out = torch.empty(max(B, 0), 8, dtype=torch.float64, device=p.device)
+    ws_bytes = lib.dfw_case_stress_summary_ws_bytes(N, B)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=p.device)
+    allow = float(allowable_pa) if allowable_pa is not None else 0.0
+    with torch.cuda.device(p.device), _prof("case_stress_summary", N * (_esz(p) + 12 + (1 if m is not None else 0)) + 8 * (B + 1) + 64 * B):
+        check(lib.dfw_case_stress_summary(p.data_ptr(), _dt(p), pos.data_ptr(), _ptr(m), cp.data_ptr(), B, N, float(root_band), allow,
+                                          int(bool(log_scale)), out.data_ptr(), ws.data_ptr(), ws_bytes, _stream(p)))
+    LAUNCH_COUNTER["kernels"] += (3 if m is not None else 4) if B > 0 else 0
+    return out
+
+
 def cast(t: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     if t.dtype == dtype:
         return t.contiguous()

@@ -229,6 +229,22 @@ def _finish(pos, normal, stress, mask, und, p, edge_rng, node_order, rng) -> dic
     }
 
 
+def geometry_case(mesh: dict, node_id_base: int = 1) -> dict:
+    """The pre-FEM content of a surface-tri mesh as the case dict ``DesignScreener.screen`` takes (node ids from
+    ``node_id_base``, faces as node ids, no normals: screening computes them)."""
+    n = mesh["num_nodes"]
+    return {"case_id": mesh["case_id"], "node_id": np.arange(n, dtype=np.int64) + node_id_base, "pos": mesh["pos"],
+            "faces": mesh["faces"].astype(np.int64) + node_id_base, "params": dict(mesh["params"])}
+
+
+def write_geometry_case(mesh: dict, out_dir: Path, node_id_base: int = 1) -> Path:
+    """Write a surface-tri mesh as a geometry case ``<out_dir>/<case_id>.npz`` (``caseio.pack_geometry_case``)."""
+    from .caseio import pack_geometry_case
+
+    c = geometry_case(mesh, node_id_base)
+    return pack_geometry_case(Path(out_dir) / f"{c['case_id']}.npz", c["case_id"], c["node_id"], c["pos"], c["faces"], c["params"])
+
+
 def write_case_files(mesh: dict, root: Path, node_id_base: int = 1) -> str:
     """Write a surface-tri mesh in the reference's on-disk case format:
     ``data/raw/fem/{id}/surface_results.npz`` (``fem.py:642-650``),

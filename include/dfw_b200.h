@@ -305,6 +305,44 @@ int dfw_stress_metrics(const void* pred, const void* target, const uint8_t* mask
                        int log_scale, int dtype, double* result, void* ws, size_t ws_bytes,
                        dfw_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Design screening (BASELINE.json config 5): what a design that has not been through FEM needs on the device.
+ *
+ * (s1) Area-weighted vertex normals of a triangulated surface: the normal block of the reference's fem.py:390-424
+ *     (restated at synth.py:146-151)
+ *         fn = cross(p1 - p0, p2 - p0);  normal[v] = sum over the incidences (f, k) with faces[f, k] == v of fn[f]
+ *     pos fp32 [N,3], faces int64 [F,3] of 0-based rows (several cases concatenated: rows of the concatenation).
+ *     Out: normal fp32 [N,3] (0 for a vertex without a face; dfw_node_features maps |n| < 1e-8 to a zero feature),
+ *     status int32 [1] (device) = faces skipped because an index was outside [0, N).  A face naming a vertex twice
+ *     contributes twice, as with numpy.bincount.
+ *     Determinism: fp32 sums in ascending incidence order 3f + k (the vertex -> incidence lists come from the canonical
+ *     CSR build of dfw_csr_build), no float atomics: bitwise identical run to run, and a vertex reads only its own faces,
+ *     so how cases are batched into one call cannot change it.  No host synchronisation.  Requires 3F, N < 2^31.
+ * ---------------------------------------------------------------------------------------- */
+size_t dfw_vertex_normals_ws_bytes(int64_t F, int64_t N);
+int dfw_vertex_normals(const float* pos, int64_t N, const int64_t* faces, int64_t F, float* normal, int32_t* status,
+                       void* ws, size_t ws_bytes, dfw_stream_t stream);
+
+/* (s2) Per-case stress summary: a segmented reduction of the model output over case_ptr (device int64 [B+1],
+ *     non-decreasing from 0 to N), one record per case - what a screening run ranks designs by, without bringing the
+ *     prediction back to the host (the reference's inference_gnn.py copies it whole, per case).
+ *     pred [N] (or [N,1]) in `dtype` holds log1p(stress) when log_scale != 0 (stress = expm1f(pred) in fp32, as in
+ *     dfw_stress_metrics), pos fp32 [N,3].  Screened rows: mask[row] != 0 when mask (uint8 [N]) is given, else
+ *     pos_y > root_band * (max_y - min_y) of the row's own case (fp64 comparison) - the rule behind the dataset's loss_mask
+ *     (fem.py:637-640, restated at synth.py:154-155).
+ *     out float64 [B,8]: [0] rows, [1] screened rows, [2] max stress over the screened rows, [3] row of that maximum within
+ *     the case (lowest row on ties; -1 when none), [4] mean stress over the screened rows, [5] max stress over all rows,
+ *     [6] screened rows with stress > allowable_pa (allowable_pa <= 0: none counted), [7] rows whose stress is not finite.
+ *     Non-finite stresses are counted in [7] only: they take no part in [2]-[6].  An empty set reports 0 in [2], [4], [5], [6].
+ *     Determinism: a case is cut into 2048-row chunks from its own first row; per chunk fp64 partial sums in a fixed
+ *     order, chunks combined in ascending order, no float atomics - a record depends on its own case only, bitwise.
+ *     The grid covers the chunks of all cases, so a large case shares a launch with small ones without serialising.
+ * ---------------------------------------------------------------------------------------- */
+size_t dfw_case_stress_summary_ws_bytes(int64_t N, int64_t B);
+int dfw_case_stress_summary(const void* pred, int dtype, const float* pos, const uint8_t* mask, const int64_t* case_ptr,
+                            int64_t B, int64_t N, double root_band, double allowable_pa, int log_scale, double* out,
+                            void* ws, size_t ws_bytes, dfw_stream_t stream);
+
 /* dtype conversion helper (weights fp32 -> bf16 copies for the bf16 path) */
 int dfw_cast(const void* src, int src_dtype, void* dst, int dst_dtype, int64_t n, dfw_stream_t stream);
 
