@@ -897,7 +897,7 @@ DwPlan dw_plan(int64_t N, int64_t Hout, int64_t k1, int64_t k2) {
     int64_t max_splits = std::max<int64_t>(1, (N + 4 * BK - 1) / (4 * BK));
     int64_t splits = std::max<int64_t>(1, std::min(want, max_splits));
     int64_t per = (N + splits - 1) / splits;
-    per = (per + BK - 1) / BK * BK;
+    per = std::max<int64_t>(BK, (per + BK - 1) / BK * BK);  // N = 0 would give per = 0 and a division by zero below
     splits = std::max<int64_t>(1, (N + per - 1) / per);
     p.splits = (int)splits;
     p.nodes_per_split = per;

@@ -590,6 +590,11 @@ __device__ __forceinline__ void epilogue_tile(const Args& p, const float* cvec, 
     uint8_t* const pre_lane = p.pre_out ? static_cast<uint8_t*>(p.pre_out) + lane_off : nullptr;
     const uint8_t* const res_lane = p.residual ? static_cast<const uint8_t*>(p.residual) + lane_off : nullptr;
     const bool has_res = res_lane != nullptr;
+    // bf16: the residual is added to the fp32 epilogue value BEFORE the one rounding to bf16, as in the classic and SIMT kernels
+    // (added after the packing it would round twice: up to 1.5 ulp).  So it is read in the thread-per-row domain, 64 contiguous
+    // bytes of the thread's own row per round.  fp32 packs exactly, so it keeps the coalesced read of the write-back domain.
+    constexpr bool kResInRow = sizeof(T) == 2;
+    const uint8_t* const res_row = (kResInRow && has_res && rok) ? static_cast<const uint8_t*>(p.residual) + (size_t)row * row_bytes : nullptr;
 
     auto load_res = [&](const uint8_t* src, uint4 (&dst)[4]) {
 #pragma unroll
@@ -718,8 +723,17 @@ __device__ __forceinline__ void epilogue_tile(const Args& p, const float* cvec, 
         const int c0 = g * 32;
         uint4 rv[ROUNDS][4];
         if (has_res) {
+            if constexpr (kResInRow) {
 #pragma unroll
-            for (int h = 0; h < ROUNDS; ++h) load_res(res_lane + (size_t)(c0 + h * SCOLS) * sizeof(T), rv[h]);
+                for (int h = 0; h < ROUNDS; ++h)
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        rv[h][j] = res_row ? *reinterpret_cast<const uint4*>(res_row + (size_t)(c0 + h * SCOLS) * sizeof(T) + j * 16)
+                                           : make_uint4(0u, 0u, 0u, 0u);
+            } else {
+#pragma unroll
+                for (int h = 0; h < ROUNDS; ++h) load_res(res_lane + (size_t)(c0 + h * SCOLS) * sizeof(T), rv[h]);
+            }
         }
         float v[32];
         if (y_in_tmem) {
@@ -759,13 +773,28 @@ __device__ __forceinline__ void epilogue_tile(const Args& p, const float* cvec, 
                 dot = fmaf(v[4 * g4 + 3], w.w, dot);
             }
         }
+        if constexpr (kResInRow) {
+            if (has_res) {
+#pragma unroll
+                for (int h = 0; h < ROUNDS; ++h)
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        Vec16<T> u;
+                        u.v = rv[h][j];
+                        float f[EPS];
+                        u.to_float(f);
+#pragma unroll
+                        for (int i = 0; i < EPS; ++i) v[h * SCOLS + j * EPS + i] += f[i];
+                    }
+            }
+        }
         if (out_lane) {
 #pragma unroll
             for (int h = 0; h < ROUNDS; ++h) {
                 uint4 pk[4];
                 pack(v + h * SCOLS, pk);
                 uint8_t* dst = out_lane + (size_t)(c0 + h * SCOLS) * sizeof(T);
-                if (has_res) stage_and_store(dst, pk, rv[h]);
+                if (has_res && !kResInRow) stage_and_store(dst, pk, rv[h]);
                 else stage_and_store(dst, pk, nullptr);
             }
         }

@@ -1,6 +1,7 @@
 """The tensor-core linear has three kernels behind one entry point: the persistent one (default), the classic one-tile-per-CTA
-kernel (shapes the persistent kernel does not take; DFW_TC_PERSIST=0 forces it) and the opt-in CTA-pair kernel (DFW_TC_PAIR=1).
-The environment switches are read once per process, so the linear parity tests are re-run in a subprocess per variant."""
+kernel (shapes the persistent kernel does not take; DFW_TC_PERSIST=0 forces it) and the opt-in CTA-pair kernel (DFW_TC_PAIR=1);
+DFW_FORCE_SIMT=1 sends every linear to the SIMT kernels.  The environment switches are read once per process, so the linear
+parity tests and the element-wise bounds of test_gpu_linear_bounds.py are re-run in a subprocess per variant."""
 import os
 import subprocess
 import sys
@@ -11,10 +12,11 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [{"DFW_TC_PERSIST": "0"}, {"DFW_TC_PAIR": "1"}], ids=["classic", "cta_pair"])
+@pytest.mark.parametrize("env", [{"DFW_TC_PERSIST": "0"}, {"DFW_TC_PAIR": "1"}, {"DFW_FORCE_SIMT": "1"}], ids=["classic", "cta_pair", "simt"])
 def test_linear_parity_suite_on_kernel_variant(env):
     e = dict(os.environ, **env)
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(REPO, "tests", "test_gpu_kernels.py"), "-m", "gpu", "-q", "-x", "-k", "linear or mlp or sage_layer",
-                        "-p", "no:cacheprovider"], cwd=REPO, env=e, capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(REPO, "tests", "test_gpu_kernels.py"),
+                        os.path.join(REPO, "tests", "test_gpu_linear_bounds.py"), "-m", "gpu", "-q", "-x", "-k", "linear or mlp or sage_layer",
+                        "-p", "no:cacheprovider"], cwd=REPO, env=e, capture_output=True, text=True, timeout=1800)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     assert " passed" in r.stdout
