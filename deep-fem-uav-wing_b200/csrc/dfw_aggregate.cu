@@ -16,7 +16,6 @@
 //    instruction-issue bound, not bandwidth bound, on a naive kernel (profiles/r01_ncu_*_v1.csv).
 // Roofline: HBM.  Algorithmic bytes per launch  A_min = 2*N*H*b + 4*E + 4*(N+1)  (DESIGN.md).
 #include <algorithm>
-#include <cstdlib>
 
 #include "dfw_common.cuh"
 
@@ -114,9 +113,12 @@ struct Acc<__nv_bfloat16> {
 //  * What bounds cfg4 now is the L2 -> SM fabric: 9.3 GB of L1 misses in 0.71 ms = 13 TB/s, the full-chip LTS
 //    cap (~6300 B/clk).  Only more on-SM reuse (explicit de-duplication of a chunk's neighbours in shared
 //    memory) can lift it further.
-//  * PIPE (batch b+1 in flight while batch b is added) is kept as a template switch: it helps at 16 warps but
-//    32 warps x one batch hide the per-block prologue (rowptr -> col -> rows) better (745 vs 956 us).
-template <typename T, int LANES, int VPL, bool HAS_ADD, bool EXACT, bool HAS_SRC, int kAggThreads, int KUDIV, bool PIPE>
+//  * 32 warps x one batch of kU rows in flight beat 16 warps x two software-pipelined batches (cfg4: 745 vs 956 us)
+//    and 32 warps x two half batches (750 us): thread-level parallelism hides the per-block prologue
+//    (rowptr -> col -> rows) best.
+constexpr int kAggThreads = 1024;
+
+template <typename T, int LANES, int VPL, bool HAS_ADD, bool EXACT, bool HAS_SRC>
 __global__ void __launch_bounds__(kAggThreads, 1) k_aggregate(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                                                               const float* __restrict__ row_scale,
                                                               const float* __restrict__ src_scale /*per SOURCE row (HAS_SRC)*/,
@@ -126,11 +128,9 @@ __global__ void __launch_bounds__(kAggThreads, 1) k_aggregate(const int32_t* __r
     using V = Vec16<T>;
     constexpr int EPV = V::N;
     constexpr int GROUPS = 32 / LANES;
-    constexpr int kU0 = VPL >= 4 ? 2 : (VPL == 2 ? 4 : 8);  // source rows per batch (8 x 16 B per lane), two batches in flight
-    constexpr int kU1 = kU0 / KUDIV < 2 ? 2 : kU0 / KUDIV;
-    constexpr int kU = kU1 < LANES ? kU1 : LANES;
+    constexpr int kU0 = VPL >= 4 ? 2 : (VPL == 2 ? 4 : 8);  // source rows per batch (8 x 16 B per lane)
+    constexpr int kU = kU0 < LANES ? kU0 : LANES;
     static_assert(LANES % kU == 0, "a column window holds whole batches");
-    static_assert(!(PIPE && HAS_SRC), "the per-batch scales live in one register set");
     __shared__ int s_next;
     __shared__ __align__(16) int s_cols[kAggThreads / 32][2][32];
     __shared__ __align__(16) float s_scl[HAS_SRC ? kAggThreads / 32 : 1][2][32];  // the columns' source scales
@@ -318,22 +318,10 @@ __global__ void __launch_bounds__(kAggThreads, 1) k_aggregate(const int32_t* __r
             }
         }
     };
-    if constexpr (PIPE) {
-        uint4 bufA[kU][VPL], bufB[kU][VPL];
-        if (nbatch > 0) issue(bufA, 0);
-        for (int b = 0; b < nbatch; b += 2) {
-            if (b + 1 < nbatch) issue(bufB, b + 1);
-            consume(bufA, b);
-            if (b + 1 >= nbatch) break;
-            if (b + 2 < nbatch) issue(bufA, b + 2);
-            consume(bufB, b + 1);
-        }
-    } else {
-        for (int b = 0; b < nbatch; ++b) {
-            uint4 buf[kU][VPL];
-            issue(buf, b);
-            consume(buf, b);
-        }
+    for (int b = 0; b < nbatch; ++b) {
+        uint4 buf[kU][VPL];
+        issue(buf, b);
+        consume(buf, b);
     }
     while (cur < nrows) flush();  // last row and trailing empty rows
   }
@@ -342,7 +330,7 @@ __global__ void __launch_bounds__(kAggThreads, 1) k_aggregate(const int32_t* __r
 // rows per group: about a dozen rows / <= 192 edges per group amortise the rowptr/col round trips of a block (the
 // dependent prologue of every block is what the 32 warps have to hide); among the candidates take the one whose
 // chunk count fills whole waves of 148 CTAs best (a 200k-row batch is only ~4 waves: 3.25 waves cost 4)
-inline int pick_rows_per_group(int64_t N, int64_t E, int lanes, int groups, int threads) {
+inline int pick_rows_per_group(int64_t N, int64_t E, int lanes, int groups) {
     const double deg = N > 0 ? (double)E / (double)N : 0.0;
     int hi = (int)(192.0 / (deg + 1.0));
     hi = std::max(1, std::min(hi, std::min(12, lanes - 1)));
@@ -350,7 +338,7 @@ inline int pick_rows_per_group(int64_t N, int64_t E, int lanes, int groups, int 
     int best = hi;
     double best_eff = -1.0;
     for (int R = hi; R >= lo; --R) {
-        const int64_t chunk_rows = (int64_t)R * groups * (threads / 32);
+        const int64_t chunk_rows = (int64_t)R * groups * (kAggThreads / 32);
         const int64_t chunks = (N + chunk_rows - 1) / chunk_rows;
         const int64_t waves = (chunks + kNumSMs - 1) / kNumSMs;
         const double eff = (double)N / ((double)waves * kNumSMs * (double)chunk_rows);
@@ -362,43 +350,29 @@ inline int pick_rows_per_group(int64_t N, int64_t E, int lanes, int groups, int 
     return best;
 }
 
-// 32 warps x one batch of kU rows in flight beat 16 warps x two software-pipelined batches (cfg4: 745 vs 956 us)
-// and 32 warps x two half batches (750 us): thread-level parallelism hides the per-block prologue best.
-constexpr int kAggThreads = 1024;
-
-template <typename T, int LANES, int VPL, int THREADS, bool PIPE>
-int launch_v(const int32_t* rowptr, const int32_t* col, const float* row_scale, const float* src_scale, const void* x,
-             const void* addend, void* out, int64_t N, int64_t E, int nvec, cudaStream_t s) {
+template <typename T, int LANES, int VPL>
+int launch(const int32_t* rowptr, const int32_t* col, const float* row_scale, const float* src_scale, const void* x,
+           const void* addend, void* out, int64_t N, int64_t E, int nvec, cudaStream_t s) {
     constexpr int GROUPS = 32 / LANES;
-    static const int env_r = [] { const char* e = getenv("DFW_AGG_R"); return e ? atoi(e) : 0; }();  // dev probe
-    const int R = env_r > 0 ? std::min(env_r, LANES - 1) : pick_rows_per_group(N, E, LANES, GROUPS, THREADS);
-    const int64_t chunk_rows = (int64_t)R * GROUPS * (THREADS / 32);
+    const int R = pick_rows_per_group(N, E, LANES, GROUPS);
+    const int64_t chunk_rows = (int64_t)R * GROUPS * (kAggThreads / 32);
     const int64_t chunks = (N + chunk_rows - 1) / chunk_rows;
     const int64_t blocks = std::min<int64_t>(chunks, kNumSMs);
     if (blocks == 0) return 0;
     const bool exact = nvec == LANES * VPL;
-#define DFW_AGG_GO(A, X, S, P)                                                                                               \
-    k_aggregate<T, LANES, VPL, A, X, S, THREADS, 1, P><<<(unsigned)blocks, THREADS, 0, s>>>(                                   \
-        rowptr, col, row_scale, src_scale, (const T*)x, (const T*)addend, (T*)out, N, nvec, R)
-    if (src_scale) {  // (the scaled gather is only used without an addend: backward of the mean; its scales live in one register set)
-        if (exact) DFW_AGG_GO(false, true, true, false); else DFW_AGG_GO(false, false, true, false);
+#define DFW_AGG_GO(A, X, S)                                                                                                  \
+    k_aggregate<T, LANES, VPL, A, X, S><<<(unsigned)blocks, kAggThreads, 0, s>>>(rowptr, col, row_scale, src_scale, (const T*)x, \
+                                                                                (const T*)addend, (T*)out, N, nvec, R)
+    if (src_scale) {  // (the scaled gather is only used without an addend: backward of the mean)
+        if (exact) DFW_AGG_GO(false, true, true); else DFW_AGG_GO(false, false, true);
     } else if (exact) {
-        if (addend) DFW_AGG_GO(true, true, false, PIPE); else DFW_AGG_GO(false, true, false, PIPE);
+        if (addend) DFW_AGG_GO(true, true, false); else DFW_AGG_GO(false, true, false);
     } else {
-        if (addend) DFW_AGG_GO(true, false, false, PIPE); else DFW_AGG_GO(false, false, false, PIPE);
+        if (addend) DFW_AGG_GO(true, false, false); else DFW_AGG_GO(false, false, false);
     }
 #undef DFW_AGG_GO
     DFW_LAUNCH_CHECK();
     return 0;
-}
-
-template <typename T, int LANES, int VPL>
-int launch(const int32_t* rowptr, const int32_t* col, const float* row_scale, const float* src_scale, const void* x,
-           const void* addend, void* out, int64_t N, int64_t E, int nvec, cudaStream_t s) {
-    static const int variant = [] { const char* e = getenv("DFW_AGG_VARIANT"); return e ? atoi(e) : 0; }();  // dev probe
-    if (variant == 1) return launch_v<T, LANES, VPL, 512, true>(rowptr, col, row_scale, src_scale, x, addend, out, N, E, nvec, s);
-    if (variant == 2) return launch_v<T, LANES, VPL, 768, false>(rowptr, col, row_scale, src_scale, x, addend, out, N, E, nvec, s);
-    return launch_v<T, LANES, VPL, kAggThreads, false>(rowptr, col, row_scale, src_scale, x, addend, out, N, E, nvec, s);
 }
 
 template <typename T>

@@ -39,7 +39,6 @@
 #include <cuda.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 
 #include "dfw_common.cuh"
@@ -677,8 +676,6 @@ extern "C" int dfw_sage_aggregate_tc(const int32_t* blk_meta, const int32_t* pla
     p.H = (int)H;
     int stages = kMaxStages;
     while (stages > 2 && carve((int)H, stages).total + 1024 > 227 * 1024) --stages;
-    static const int env_stages = [] { const char* e = getenv("DFW_AGGTC_STAGES"); return e ? atoi(e) : 0; }();  // dev probe
-    if (env_stages >= 2 && env_stages < stages) stages = env_stages;
     p.stages = stages;
     const size_t smem = carve((int)H, stages).total + 1024;
     p.out = static_cast<uint8_t*>(out);

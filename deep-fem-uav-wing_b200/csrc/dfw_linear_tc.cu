@@ -75,27 +75,13 @@ __host__ __device__ inline Smem carve(bool tf32, int Npad, int stages, int out_b
     return s;
 }
 
-#ifdef DFW_TC_PROBE
-__device__ long long* g_probe = nullptr;  // [96] stamps of one mid-grid CTA (tools/tc_timeline.py)
-__device__ __forceinline__ void probe(int slot) {
-    if (g_probe && blockIdx.x == gridDim.x / 2) {
-        long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        g_probe[slot] = t;
-    }
-}
-#define PROBE(slot) probe(slot)
-#else
-#define PROBE(slot)
-#endif
-
 template <typename T, bool TF32>
 __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ Maps maps, const Args p) {
     constexpr int EPC = kChunkBytes / (int)sizeof(T);  // elements (columns) per 128-byte epilogue box: 32 fp32 / 64 bf16
     // Main-loop K chunk: 128 B (SWIZZLE_128B) for bf16, 64 B (SWIZZLE_64B) for fp32.  The fp32 stage holds four
     // tiles (a_hi, a_lo, w_hi, w_lo); with 64-byte chunks a stage is 32 KB, three stages fit in < 110 KB and TWO
     // CTAs share an SM, so the epilogue of one tile overlaps the main loop of another (one CTA per SM leaves the
-    // epilogue latency - ~7 us per tile - fully exposed; measured with the clock probes of tools/tc_timeline.py).
+    // epilogue latency - ~7 us per tile - fully exposed; measured with %globaltimer probes).
     constexpr int CB = TF32 ? 64 : 128;
     constexpr int KPC = CB / (int)sizeof(T);           // K elements per chunk
     extern __shared__ uint8_t smem_raw[];
@@ -112,23 +98,11 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
     uint64_t* res_full = accum_full + 1;
     uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(res_full + 1);
 
-    if (threadIdx.x == 0) PROBE(65);  // kernel entry
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t m_base = (int64_t)blockIdx.x * kTileM;  // CTAs padding the grid to whole clusters own an empty tile
+    const int64_t m_base = (int64_t)blockIdx.x * kTileM;
     const int total_chunks = p.chunks[0] + p.chunks[1];
-    // Thread-block cluster: every CTA needs the SAME weight chunks, and at K*Hout*(4+4) bytes per 128-row tile they
-    // are two thirds of what a CTA pulls through the L2 fabric (ncu r01: 1.24 GB of L2 traffic per launch, 8.8 TB/s
-    // of a ~13 TB/s cap, for 0.4 GB of DRAM traffic).  So CTA 0 of the cluster fetches each weight chunk ONCE and
-    // multicasts it to all peers; every CTA loads its own activation rows.  A stage is refilled only when every CTA
-    // of the cluster has retired the MMAs that read it (the commits are multicast to every peer's `empty` barrier).
-    // MEASURED (r01, cfg2 fwd, L2 flushed): cluster 1 / 2 / 4 = 146 / 155 / 159 us - the lock-step between the CTAs costs
-    // more than the L2 reads save, because a tile is bound by the round trip of its few smem stages and by the
-    // tensor pipe (64 MMAs x ~140 clk per tile, shared by the two resident CTAs), not by the fabric.  The launcher
-    // therefore uses clusters of 1; DFW_TC_CLUSTER=2|4 keeps the path testable.
-    const uint32_t csize = cluster_nctarank(), crank = csize > 1 ? cluster_ctarank() : 0u;
-    const uint16_t cmask = (uint16_t)((1u << csize) - 1u);
-
     // One chunk = one pipeline stage: the activation box of this CTA's rows plus the weight boxes of the same K range.
+    // Every CTA loads its own weights: multicasting them over a thread-block cluster was measured slower (DESIGN.md section 4).
     const uint32_t stage_tx = (uint32_t)(kTileM * CB + p.Npad * CB * (TF32 ? 2 : 1));
     auto issue_chunk = [&](int c, int stage) {
         const int seg = c >= p.chunks[0];
@@ -136,19 +110,14 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
         uint8_t* st = smem + (size_t)stage * L.stage_bytes;
         mbar_arrive_expect_tx(&full[stage], stage_tx);
         tma_load_2d(st + L.a_hi, &maps.a[seg], &full[stage], kc, (int)m_base);
-        if (csize == 1) {
-            tma_load_2d(st + L.w_hi, &maps.w_hi[seg], &full[stage], kc, 0);
-            if (TF32) tma_load_2d(st + L.w_lo, &maps.w_lo[seg], &full[stage], kc, 0);
-        } else if (crank == 0) {
-            tma_load_2d_mc(st + L.w_hi, &maps.w_hi[seg], &full[stage], kc, 0, cmask);
-            if (TF32) tma_load_2d_mc(st + L.w_lo, &maps.w_lo[seg], &full[stage], kc, 0, cmask);
-        }
+        tma_load_2d(st + L.w_hi, &maps.w_hi[seg], &full[stage], kc, 0);
+        if (TF32) tma_load_2d(st + L.w_lo, &maps.w_lo[seg], &full[stage], kc, 0);
     };
     int prefilled = 0;  // producer thread: chunks requested before the setup barrier
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < p.stages; ++s) {
             mbar_init(&full[s], 1);
-            mbar_init(&empty[s], csize);
+            mbar_init(&empty[s], 1);
             mbar_init(&conv[s], 128);
         }
         mbar_init(accum_full, 1);
@@ -156,11 +125,9 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         // The first ring of loads needs neither TMEM nor the per-column constants: request it NOW, so the ~1 us of DRAM
         // latency runs under the rest of the setup (TMEM allocation, constant loads, the block-wide barrier) instead of
-        // after it.  (In a cluster the peers' barriers must exist first: no early start there.)
-        if (csize == 1) {
-            prefilled = total_chunks < p.stages ? total_chunks : p.stages;
-            for (int c = 0; c < prefilled; ++c) issue_chunk(c, c);
-        }
+        // after it.
+        prefilled = total_chunks < p.stages ? total_chunks : p.stages;
+        for (int c = 0; c < prefilled; ++c) issue_chunk(c, c);
         prefetch_tmap(&maps.w_hi[0]);
         if (p.chunks[1]) {
             prefetch_tmap(&maps.a[1]);
@@ -184,9 +151,7 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
     fence_tc_before();
     __syncthreads();
     fence_tc_after();
-    if (csize > 1) cluster_sync_all();  // peers' barriers exist before anything is multicast to them
     const uint32_t tmem_base = *tmem_ptr;
-    if (threadIdx.x == 0) PROBE(0);
 
     if (warp == 0) {
         // ===== TMA producer =====
@@ -227,7 +192,6 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
             for (int c = 0; c < total_chunks; ++c) {
                 mbar_wait(TF32 ? &conv[stage] : &full[stage], phase);
                 fence_tc_after();
-                if (c < 20) PROBE(1 + c);  // operands of chunk c ready
                 const uint32_t st = smem_u32(smem + (size_t)stage * L.stage_bytes);
 #pragma unroll
                 for (int k = 0; k < CB / 32; ++k) {  // UMMA_K = 32 bytes (16 bf16 / 8 tf32); +32 B = +2 in the address field
@@ -258,9 +222,7 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
                     }
                     accumulate = 1u;
                 }
-                // frees the smem stage once these MMAs have read it (in a cluster: tells every peer)
-                if (csize == 1) umma_commit(&empty[stage]);
-                else umma_commit_mc(&empty[stage], cmask);
+                umma_commit(&empty[stage]);  // frees the smem stage once these MMAs have read it
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
             }
             umma_commit(accum_full);
@@ -273,7 +235,6 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
             uint32_t phase = 0;
             for (int c = 0; c < total_chunks; ++c) {
                 mbar_wait(&full[stage], phase);
-                if (et == 0 && c < 20) PROBE(21 + c);  // TMA data of chunk c landed
                 uint8_t* st = smem + (size_t)stage * L.stage_bytes;
                 float4* hi = reinterpret_cast<float4*>(st + L.a_hi);
                 float4* lo = reinterpret_cast<float4*>(st + L.a_lo);
@@ -290,7 +251,6 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
 
         mbar_wait(accum_full, 0);
         fence_tc_after();
-        if (et == 0) PROBE(41);  // accumulator complete
         const int q = warp & 3;  // TMEM lane quarter this warp may access
         const int r_in_tile = q * 32 + lane;
         const int64_t row = m_base + r_in_tile;
@@ -409,7 +369,6 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
             tmem_st_wait();
             mean = s / (float)H;
         }
-        if (et == 0) PROBE(43);  // pass 1 (accumulators combined, pre-activation staged + stored)
         // ---- pass 2: variance around the mean (two-pass, like torch) ----
         if (ln) {
             float qs = 0.f;
@@ -433,10 +392,8 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
                 p.ln_stats[2 * row + 1] = rstd;
             }
         }
-        if (et == 0) PROBE(44);  // pass 2 (variance)
         // ---- pass 3: normalise, ReLU, dropout, row-dot, residual, store ----
         if (p.residual) mbar_wait(res_full, 0);
-        if (et == 0) PROBE(45);  // residual tile in smem
         float dot = 0.f;
         {
             const bool sum_here = !y_in_tmem && regions > 1;
@@ -450,7 +407,6 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
                 const uint8_t* rbox = smem + L.res + (size_t)ob * kTileM * kChunkBytes;
                 float v[32];
                 tmem_ld_wait(ra);
-                if (et == 0 && g < 4) PROBE(50 + 4 * g);  // TMEM values here
                 if (sum_here) {
                     tmem_ld_wait(rb);
 #pragma unroll
@@ -520,19 +476,14 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
                         }
                     }
                 }
-                if (et == 0 && g < 4) PROBE(51 + 4 * g);  // math done
                 if (p.out) {
                     if (c0 % EPC == 0) box = acquire_box();
-                    if (et == 0 && g < 4) PROBE(49 + 4 * g);  // box acquired
                     stage_row(box, h * 32, v);
                     if ((c0 + 32) % EPC == 0) release_box(p.out, box, ob * EPC);
                 }
-                if (et == 0 && g < 4) PROBE(52 + 4 * g);  // staged + store issued
             }
         }
         if (p.rowdot_out && rok) p.rowdot_out[row] = dot + (p.rowdot_b ? __ldg(p.rowdot_b) : 0.f);
-        if (et == 0) PROBE(46);  // pass 3 done
-        if (et == 0) PROBE(47);
     }
 
     fence_tc_before();
@@ -541,14 +492,12 @@ __global__ void __launch_bounds__(kThreads) k_linear_tc(const __grid_constant__ 
         fence_tc_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols) : "memory");
     }
-    if (csize > 1) cluster_sync_all();  // no CTA leaves while a peer may still signal its barriers
-    if (threadIdx.x == 0) PROBE(48);
 }
 
 // The three epilogue passes of one 128-row tile for ONE thread (= tile row `q*32 + lane`, whose accumulator lives in TMEM lane
 // `q*32 + lane` from column `t_row`): y = (acc + bias) * row_scale, LayerNorm, ReLU, dropout, row-dot, residual, stores through the
-// warp's private staging slice.  Shared by the persistent kernels (k_linear_tcp, k_linear_tc2).
-// Written lean on purpose: tools/lin_knock.py + the ncu source page showed the epilogue warps, not the main loop, pacing the
+// warp's private staging slice.  Used by the persistent kernel k_linear_tcp.
+// Written lean on purpose: knock-out timing (DESIGN.md section 4) + the ncu source page showed the epilogue warps, not the main loop, pacing the
 // persistent kernel (epilogue alone 114 us of the 134 us SAGE forward;
 // main loop alone 77 us): ~6.4k warp instructions per tile and warp at ~0.2 IPC, a third of them address / predicate / branch
 // overhead of the write-back (64-bit row bound checks and a reconvergence region per store, register copies of the prefetched
@@ -648,7 +597,7 @@ __device__ __forceinline__ void epilogue_tile(const Args& p, const float* cvec, 
         }
     };
     auto load_acc = [&](int c0, float* v) {  // hi*hi + cross terms, summed in round-to-nearest fp32 (see tmem_combine)
-        if (TF32 && p.nacc != 0) {
+        if (TF32) {
             uint32_t ra[32], rb[32];
             tmem_ld32_issue(t_row + c0, ra);
             tmem_ld32_issue(t_row + p.Npad + c0, rb);
@@ -898,8 +847,7 @@ __global__ void __launch_bounds__(kPThreads, 1) k_linear_tcp(const __grid_consta
       if (warp == 0) {
         // ===== TMA producer =====
         if (lane == 0) {
-            const bool ld_a = !(p.knock & 16), ld_w = !(p.knock & 4);
-            const uint32_t stage_tx = (uint32_t)((ld_a ? kTileM * 128 : 0) + (ld_w ? p.Npad * 128 * (TF32 ? 2 : 1) : 0));
+            const uint32_t stage_tx = (uint32_t)(kTileM * 128 + p.Npad * 128 * (TF32 ? 2 : 1));
             int stage = 0;
             uint32_t phase = 0;
             for (int i = 0; i < nmine; ++i) {
@@ -909,11 +857,10 @@ __global__ void __launch_bounds__(kPThreads, 1) k_linear_tcp(const __grid_consta
                     const int kc = (seg ? c - p.chunks[0] : c) * KPC;
                     mbar_wait(&empty[stage], phase ^ 1);
                     uint8_t* st = smem + (size_t)stage * L.stage_bytes;
-                    if (stage_tx) mbar_arrive_expect_tx(&full[stage], stage_tx);
-                    else mbar_arrive(&full[stage]);
-                    if (ld_a) tma_load_2d(st + L.a_hi, &maps.a[seg], &full[stage], kc, m_base);
-                    if (ld_w) tma_load_2d(st + L.w_hi, &maps.w_hi[seg], &full[stage], kc, 0);
-                    if (TF32 && ld_w) tma_load_2d(st + L.w_lo, &maps.w_lo[seg], &full[stage], kc, 0);
+                    mbar_arrive_expect_tx(&full[stage], stage_tx);
+                    tma_load_2d(st + L.a_hi, &maps.a[seg], &full[stage], kc, m_base);
+                    tma_load_2d(st + L.w_hi, &maps.w_hi[seg], &full[stage], kc, 0);
+                    if (TF32) tma_load_2d(st + L.w_lo, &maps.w_lo[seg], &full[stage], kc, 0);
                     if (++stage == p.stages) { stage = 0; phase ^= 1; }
                 }
             }
@@ -939,20 +886,12 @@ __global__ void __launch_bounds__(kPThreads, 1) k_linear_tcp(const __grid_consta
                     const uint32_t st = smem_u32(smem + (size_t)stage * L.stage_bytes);
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {  // UMMA_K = 32 bytes
-                        if (p.knock & 2) break;
                         const uint64_t a_hi = dbase + ((st + L.a_hi + k * 32) >> 4);
                         const uint64_t w_hi = dbase + ((st + L.w_hi + k * 32) >> 4);
                         if (TF32) {
                             const uint64_t a_lo = dbase + ((st + L.a_lo + k * 32) >> 4);
-                            if (p.nacc != 0) {
-                                umma<TF32>(d_tmem, a_hi, w_hi, idesc2, accumulate);                   // main = a_hi.w_hi | cross = a_hi.w_lo
-                                umma<TF32>(d_tmem + (uint32_t)p.Npad, a_lo, w_hi, idesc, 1u);         // cross += a_lo.w_hi
-                            } else {  // dev probe (DFW_TC_MERGE=1): all three products into ONE accumulator
-                                const uint64_t w_lo = dbase + ((st + L.w_lo + k * 32) >> 4);
-                                umma<TF32>(d_tmem, a_lo, w_hi, idesc, accumulate);
-                                umma<TF32>(d_tmem, a_hi, w_lo, idesc, 1u);
-                                umma<TF32>(d_tmem, a_hi, w_hi, idesc, 1u);
-                            }
+                            umma<TF32>(d_tmem, a_hi, w_hi, idesc2, accumulate);            // main = a_hi.w_hi | cross = a_hi.w_lo
+                            umma<TF32>(d_tmem + (uint32_t)p.Npad, a_lo, w_hi, idesc, 1u);  // cross += a_lo.w_hi
                         } else {
                             umma<TF32>(d_tmem, a_hi, w_hi, idesc, accumulate);
                         }
@@ -978,10 +917,8 @@ __global__ void __launch_bounds__(kPThreads, 1) k_linear_tcp(const __grid_consta
                 uint8_t* st = smem + (size_t)stage * L.stage_bytes;
                 const float4* hi = reinterpret_cast<const float4*>(st + L.a_hi);
                 float4* lo = reinterpret_cast<float4*>(st + L.a_lo);
-                if (!(p.knock & 1)) {
 #pragma unroll
-                    for (int j = 0; j < (kTileM * 128 / 16) / 128; ++j) lo[ct + j * 128] = tf32_lo(hi[ct + j * 128]);
-                }
+                for (int j = 0; j < (kTileM * 128 / 16) / 128; ++j) lo[ct + j * 128] = tf32_lo(hi[ct + j * 128]);
                 fence_proxy_async();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&conv[stage]);
@@ -1002,10 +939,8 @@ __global__ void __launch_bounds__(kPThreads, 1) k_linear_tcp(const __grid_consta
             fence_tc_after();
             const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)ab * buf_cols;
 
-            if (!(p.knock & 8)) {
-                if (m_base + kTileM <= p.N) epilogue_tile<T, TF32, true>(p, cvec, HP, slice, t_row, m_base, q, lane);
-                else epilogue_tile<T, TF32, false>(p, cvec, HP, slice, t_row, m_base, q, lane);
-            }
+            if (m_base + kTileM <= p.N) epilogue_tile<T, TF32, true>(p, cvec, HP, slice, t_row, m_base, q, lane);
+            else epilogue_tile<T, TF32, false>(p, cvec, HP, slice, t_row, m_base, q, lane);
             fence_tc_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(&acc_empty[ab]);
@@ -1017,273 +952,6 @@ __global__ void __launch_bounds__(kPThreads, 1) k_linear_tcp(const __grid_consta
     if (warp == 2) {
         fence_tc_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols) : "memory");
-    }
-}
-
-// =====================================================================================================================
-// CTA-pair variant (cta_group::2): two CTAs of a cluster (one TPC) issue ONE tcgen05.mma over their two 128-row tiles
-// (M = 256); the B operand (weights) is split by output columns between the two CTAs, so each CTA holds HALF of the weight
-// bytes - small enough to stay RESIDENT in shared memory for the whole kernel (fp32 H = 128, K = 256: 128 KB per CTA for hi + lo).
-// Per tile only the activations stream through the TMA ring (k_linear_tc re-fetches 2/3 of every stage - the weights - from L2
-// for every 128 rows; tools/probes/tma_rate_probe.cu and the ncu captures show that stream, not HBM, pacing its main loop).
-//   leader CTA (rank 0): its MMA thread issues for both; tcgen05.commit multicasts to both CTAs' barriers
-//   both CTAs: own TMA producer (own activation tile), own converters (fp32 a_lo) which signal the LEADER's `ready` barrier
-//   (remote mbarrier arrive), own two epilogue warpgroups draining their own TMEM (double-buffered accumulators), which release
-//   the accumulator buffer on the leader's `acc_empty` barrier.
-// fp32: three MMAs per k-step (a_hi.w_hi -> main; a_lo.w_hi, a_hi.w_lo -> cross), each M = 256, N = Npad.
-// =====================================================================================================================
-constexpr int k2Threads = 512;
-constexpr int k2StagesMax = 6;
-
-struct Layout2 {
-    uint32_t cb, w_chunk, w_lo_off, w_bytes, a_hi, a_lo, stage_bytes, stages_off, staging, cvec, bars, total;
-};
-__host__ __device__ inline Layout2 carve2(bool tf32, int Npad, int Hout, int total_chunks, int stages) {
-    Layout2 L;
-    L.cb = tf32 ? 64u : 128u;                                   // K bytes per chunk (fp32: SWIZZLE_64B, bf16: SWIZZLE_128B)
-    const uint32_t wh = (uint32_t)(Npad / 2) * L.cb;            // this CTA's half of the weight rows, one chunk
-    L.w_lo_off = (wh + 1023u) / 1024u * 1024u;
-    L.w_chunk = tf32 ? 2 * L.w_lo_off : L.w_lo_off;
-    L.w_bytes = L.w_chunk * (uint32_t)total_chunks;
-    const uint32_t a = kTileM * L.cb;
-    L.a_hi = 0;
-    L.a_lo = a;
-    L.stage_bytes = tf32 ? 2 * a : a;
-    L.stages_off = L.w_bytes;
-    L.staging = L.stages_off + L.stage_bytes * (uint32_t)stages;
-    L.cvec = L.staging + 8u * 2048u;
-    L.bars = L.cvec + 4u * (uint32_t)((Hout + 31) / 32 * 32) * 4u;
-    L.total = L.bars + 8u * (3 * k2StagesMax + 5) + 16u;
-    return L;
-}
-
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t local_addr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {  // barrier also signalled by the peer CTA
-    const uint32_t addr = smem_u32(bar);
-    uint32_t ok, spins = 0;
-    do {
-        asm volatile(
-            "{\n.reg .pred p;\nmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-            : "=r"(ok)
-            : "r"(addr), "r"(parity)
-            : "memory");
-        if (!ok && ++spins > (1u << 24)) {
-            printf("dfw_linear_tc2: mbarrier wait timed out (block %d thread %d bar %u parity %u)\n", blockIdx.x, threadIdx.x, addr, parity);
-            __trap();
-        }
-    } while (!ok);
-}
-template <bool TF32>
-__device__ __forceinline__ void umma2(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if constexpr (TF32) {
-        asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n}\n" ::"r"(d_tmem), "l"(adesc),
-                     "l"(bdesc), "r"(idesc), "r"(accumulate)
-                     : "memory");
-    } else {
-        asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(d_tmem), "l"(adesc),
-                     "l"(bdesc), "r"(idesc), "r"(accumulate)
-                     : "memory");
-    }
-}
-__device__ __forceinline__ void umma2_commit_mc(uint64_t* bar) {  // arrive on this barrier offset in BOTH CTAs once the MMAs issued so far retire
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
-
-template <typename T, bool TF32>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(k2Threads, 1) k_linear_tc2(const __grid_constant__ Maps maps, const Args p, const int num_pairs) {
-    constexpr int CB = TF32 ? 64 : 128;
-    constexpr int KPC = CB / (int)sizeof(T);
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    const int total_chunks = p.chunks[0] + p.chunks[1];
-    const Layout2 L = carve2(TF32, p.Npad, p.Hout, total_chunks, p.stages);
-    const int HP = (p.Hout + 31) / 32 * 32;
-    float* cvec = reinterpret_cast<float*>(smem + L.cvec);
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem + L.bars);  // [stages] local: this CTA's activation chunk landed
-    uint64_t* empty = full + k2StagesMax;                          // [stages] both: MMAs that read the stage retired (multicast commit)
-    uint64_t* ready = empty + k2StagesMax;                         // [stages] LEADER's: both CTAs' operands of the stage are ready
-    uint64_t* acc_full = ready + k2StagesMax;                      // [2] both (multicast commit)
-    uint64_t* acc_empty = acc_full + 2;                            // [2] LEADER's: both CTAs' epilogues drained the buffer
-    uint64_t* w_full = acc_empty + 2;                              // local: this CTA's resident weights landed
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(w_full + 1);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int pair0 = (int)blockIdx.x >> 1, npc = (int)gridDim.x >> 1;  // this cluster's first tile pair, number of clusters
-    const int nmine = pair0 < num_pairs ? (num_pairs - 1 - pair0) / npc + 1 : 0;
-    const int regions = TF32 ? 2 : 1;
-    const uint32_t buf_cols = (uint32_t)(regions * p.Npad);
-    const int ready_count = TF32 ? 8 : 2;
-
-    if (warp == 0 && lane == 0) {
-        for (int s = 0; s < p.stages; ++s) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], 1);
-            mbar_init(&ready[s], ready_count);
-        }
-        for (int b = 0; b < 2; ++b) {
-            mbar_init(&acc_full[b], 1);
-            mbar_init(&acc_empty[b], 8);
-        }
-        mbar_init(w_full, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        prefetch_tmap(&maps.a[0]);
-        prefetch_tmap(&maps.w_hi[0]);
-    }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr)), "r"((uint32_t)p.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    for (int c = threadIdx.x; c < p.Hout; c += k2Threads) {
-        cvec[c] = p.bias ? __ldg(p.bias + c) : 0.f;
-        cvec[HP + c] = p.gamma ? __ldg(p.gamma + c) : 1.f;
-        cvec[2 * HP + c] = p.beta ? __ldg(p.beta + c) : 0.f;
-        cvec[3 * HP + c] = p.rowdot_w ? __ldg(p.rowdot_w + c) : 0.f;
-    }
-    fence_tc_before();
-    __syncthreads();
-    cluster_sync_all();  // both CTAs' barriers exist before anything is signalled across the pair
-    fence_tc_after();
-    const uint32_t tmem_base = *tmem_ptr;
-    const uint32_t ready_leader = map_to_cta(smem_u32(ready), 0);        // + 8 * stage
-    const uint32_t acc_empty_leader = map_to_cta(smem_u32(acc_empty), 0);  // + 8 * buffer
-
-    if (warp == 0) {
-        // ===== TMA producer: the resident weight half once, then this CTA's activation tiles =====
-        if (lane == 0) {
-            const int half = p.Npad / 2;
-            mbar_arrive_expect_tx(w_full, (uint32_t)(total_chunks * half * CB * (TF32 ? 2 : 1)));
-            for (int c = 0; c < total_chunks; ++c) {
-                const int seg = c >= p.chunks[0];
-                const int kc = (seg ? c - p.chunks[0] : c) * KPC;
-                uint8_t* wc = smem + (size_t)c * L.w_chunk;
-                tma_load_2d(wc, &maps.w_hi[seg], w_full, kc, (int)rank * half);
-                if (TF32) tma_load_2d(wc + L.w_lo_off, &maps.w_lo[seg], w_full, kc, (int)rank * half);
-            }
-            int stage = 0;
-            uint32_t phase = 0;
-            for (int i = 0; i < nmine; ++i) {
-                const int m_base = (2 * (pair0 + i * npc) + (int)rank) * kTileM;
-                for (int c = 0; c < total_chunks; ++c) {
-                    const int seg = c >= p.chunks[0];
-                    const int kc = (seg ? c - p.chunks[0] : c) * KPC;
-                    mbar_wait(&empty[stage], phase ^ 1);
-                    uint8_t* st = smem + L.stages_off + (size_t)stage * L.stage_bytes;
-                    mbar_arrive_expect_tx(&full[stage], (uint32_t)(kTileM * CB));
-                    tma_load_2d(st + L.a_hi, &maps.a[seg], &full[stage], kc, m_base);
-                    if (++stage == p.stages) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ===== MMA issuer (leader CTA only) =====
-        if (lane == 0 && rank == 0) {
-            const uint32_t fmt = TF32 ? 2u : 1u;
-            // M = 256 (both CTAs' 128 rows), N = Npad (each CTA supplies Npad / 2 weight rows)
-            const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(p.Npad >> 3) << 17) | ((uint32_t)((2 * kTileM) >> 4) << 24);
-            const uint64_t dbase = make_desc_k<CB>(0);
-            int stage = 0;
-            uint32_t phase = 0;
-            for (int i = 0; i < nmine; ++i) {
-                const int ab = i & 1;
-                mbar_wait_cluster(&acc_empty[ab], (uint32_t)(((i >> 1) & 1) ^ 1));
-                fence_tc_after();
-                const uint32_t d_main = tmem_base + (uint32_t)ab * buf_cols;
-                const uint32_t d_cross = d_main + (uint32_t)p.Npad;
-                uint32_t acc_m = 0, acc_c = 0;
-                for (int c = 0; c < total_chunks; ++c) {
-                    mbar_wait_cluster(&ready[stage], phase);
-                    fence_tc_after();
-                    const uint32_t st = smem_u32(smem + L.stages_off + (size_t)stage * L.stage_bytes);
-                    const uint32_t wc = smem_u32(smem + (size_t)c * L.w_chunk);
-#pragma unroll
-                    for (int k = 0; k < CB / 32; ++k) {
-                        const uint64_t a_hi = dbase + ((st + L.a_hi + k * 32) >> 4);
-                        const uint64_t w_hi = dbase + ((wc + k * 32) >> 4);
-                        umma2<TF32>(d_main, a_hi, w_hi, idesc, acc_m);
-                        acc_m = 1u;
-                        if (TF32) {
-                            const uint64_t a_lo = dbase + ((st + L.a_lo + k * 32) >> 4);
-                            const uint64_t w_lo = dbase + ((wc + L.w_lo_off + k * 32) >> 4);
-                            umma2<TF32>(d_cross, a_lo, w_hi, idesc, acc_c);
-                            umma2<TF32>(d_cross, a_hi, w_lo, idesc, 1u);
-                            acc_c = 1u;
-                        }
-                    }
-                    umma2_commit_mc(&empty[stage]);
-                    if (++stage == p.stages) { stage = 0; phase ^= 1; }
-                }
-                umma2_commit_mc(&acc_full[ab]);
-            }
-        }
-    } else if (warp == 3) {
-        // ===== relay (bf16): this CTA's chunk landed -> the leader's `ready` barrier =====
-        if (!TF32 && lane == 0) {
-            mbar_wait(w_full, 0);
-            int stage = 0;
-            uint32_t phase = 0;
-            const int nchunks = nmine * total_chunks;
-            for (int g = 0; g < nchunks; ++g) {
-                mbar_wait(&full[stage], phase);
-                mbar_arrive_cluster(ready_leader + 8u * (uint32_t)stage);
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp >= 12) {
-        // ===== converters (fp32): a_lo = a - trunc_tf32(a); then this CTA's share of the stage is ready =====
-        if (TF32) {
-            const int ct = threadIdx.x - 384;
-            mbar_wait(w_full, 0);
-            int stage = 0;
-            uint32_t phase = 0;
-            const int nchunks = nmine * total_chunks;
-            for (int g = 0; g < nchunks; ++g) {
-                mbar_wait(&full[stage], phase);
-                uint8_t* st = smem + L.stages_off + (size_t)stage * L.stage_bytes;
-                const float4* hi = reinterpret_cast<const float4*>(st + L.a_hi);
-                float4* lo = reinterpret_cast<float4*>(st + L.a_lo);
-#pragma unroll
-                for (int j = 0; j < (kTileM * CB / 16) / 128; ++j) lo[ct + j * 128] = tf32_lo(hi[ct + j * 128]);
-                fence_proxy_async();
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cluster(ready_leader + 8u * (uint32_t)stage);
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp >= 4) {
-        // ===== epilogue warpgroups (own TMEM, own tile): WG0 takes even tile pairs, WG1 odd ones =====
-        const int wg = (warp - 4) >> 2;
-        const int q = warp & 3;
-        uint8_t* slice = smem + L.staging + (size_t)(warp - 4) * 2048;
-        for (int i = wg; i < nmine; i += 2) {
-            const int64_t m_base = (int64_t)(2 * (pair0 + i * npc) + (int)rank) * kTileM;
-            const int ab = i & 1;
-            mbar_wait(&acc_full[ab], (uint32_t)((i >> 1) & 1));
-            fence_tc_after();
-            const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)ab * buf_cols;
-            if (m_base + kTileM <= p.N) epilogue_tile<T, TF32, true>(p, cvec, HP, slice, t_row, m_base, q, lane);
-            else epilogue_tile<T, TF32, false>(p, cvec, HP, slice, t_row, m_base, q, lane);
-            fence_tc_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(acc_empty_leader + 8u * (uint32_t)ab);
-        }
-    }
-
-    fence_tc_before();
-    __syncthreads();
-    cluster_sync_all();  // no CTA leaves (or frees TMEM) while its peer may still read its shared memory or signal its barriers
-    if (warp == 2) {
-        fence_tc_after();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols) : "memory");
     }
 }
 
@@ -1322,16 +990,6 @@ __global__ void k_prep_weight(const PrepArgs a, int transpose, int split) {
         }
     }
 }
-
-#ifdef DFW_TC_PROBE
-}  // namespace tc
-}  // namespace dfw
-extern "C" int dfw_tc_set_probe(long long* dev_buf) {
-    return cudaMemcpyToSymbol(dfw::tc::g_probe, &dev_buf, sizeof(dev_buf)) == cudaSuccess ? 0 : 1;
-}
-namespace dfw {
-namespace tc {
-#endif
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -1434,57 +1092,6 @@ int linear_tc_launch(const void* a1, const void* w1, int64_t k1, const void* a2,
         DFW_LAUNCH_CHECK();
     }
 
-    // ---- CTA-pair variant (cta_group::2, resident weight halves) where the weights fit ----
-    {
-        // Measured (tools/lin_ab.py, profiles/r02_linear_pair_ab.json): correct (all parity tests pass with it forced on) but SLOWER
-        // than the one-CTA kernels - fp32 H=128 SAGE forward 210 vs 140 us, bf16 H=256 1127 vs 912 us: with the weights resident
-        // only 4 x 16 KB activation stages fit, and every 64-byte chunk pays two cross-SM handshakes (remote mbarrier arrive,
-        // cluster-scope wait, multicast commit: ~5 us per stage round trip).  Kept as an opt-in (DFW_TC_PAIR=1) with its tests.
-        static const int env_pair = [] { const char* e = getenv("DFW_TC_PAIR"); return e ? atoi(e) : 0; }();
-        const int Npad = (int)((Hout + 15) / 16 * 16);
-        const int regions = tf32 ? 2 : 1;
-        const int64_t tiles64 = (args.N + kTileM - 1) / kTileM;
-        const int cb = tf32 ? 64 : 128;
-        const int ch0 = (int)((k1 * e + cb - 1) / cb), ch1 = a2 ? (int)((k2 * e + cb - 1) / cb) : 0;
-        if (env_pair && Npad % 32 == 0 && 2 * regions * Npad <= 512 && Hout % 32 == 0 && tiles64 >= 4) {
-            int stages = k2StagesMax;
-            while (stages > 2 && carve2(tf32, Npad, (int)Hout, ch0 + ch1, stages).total + 1024 > 227 * 1024) --stages;
-            if (carve2(tf32, Npad, (int)Hout, ch0 + ch1, stages).total + 1024 <= 227 * 1024 && (stages >= 3 || env_pair == 2)) {
-                Maps pm;
-                memset(&pm, 0, sizeof(pm));
-                args.Npad = Npad;
-                args.nacc = 1;
-                int cols = 32;
-                while (cols < 2 * regions * Npad) cols <<= 1;
-                args.tmem_cols = cols;
-                args.chunks[0] = ch0;
-                args.chunks[1] = ch1;
-                args.stages = stages;
-                const int mm = tf32 ? kMapSw64 : kMapSw128;
-                const void* as2[2] = {a1, a2};
-                for (int i = 0; i < (a2 ? 2 : 1); ++i) {
-                    if (make_map(&pm.a[i], as2[i], args.N, ks[i], e, kTileM, mm)) return 1;
-                    if (make_map(&pm.w_hi[i], wuse[i], Hout, ks[i], e, Npad / 2, mm)) return 1;
-                    if (tf32 && make_map(&pm.w_lo[i], lo[i], Hout, ks[i], e, Npad / 2, mm)) return 1;
-                }
-                const size_t psmem = carve2(tf32, Npad, (int)Hout, ch0 + ch1, stages).total + 1024;
-                const int num_pairs = (int)((tiles64 + 1) / 2);
-                const unsigned grid = 2u * (unsigned)std::min<int>(num_pairs, kNumSMs / 2);
-                if (tf32) {
-                    auto kern = k_linear_tc2<float, true>;
-                    DFW_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
-                    kern<<<grid, k2Threads, psmem, s>>>(pm, args, num_pairs);
-                } else {
-                    auto kern = k_linear_tc2<__nv_bfloat16, false>;
-                    DFW_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
-                    kern<<<grid, k2Threads, psmem, s>>>(pm, args, num_pairs);
-                }
-                DFW_LAUNCH_CHECK();
-                return 0;
-            }
-        }
-    }
-
     // ---- persistent variant (one CTA per SM, 128-byte K chunks, double-buffered accumulator) where its TMEM budget fits ----
     {
         // Measured A/B (tools/lin_ab.py, profiles/r02_linear_persistent_ab.json; us, classic -> persistent, L2 flushed):
@@ -1502,10 +1109,7 @@ int linear_tc_launch(const void* a1, const void* w1, int64_t k1, const void* a2,
             Maps pm;
             memset(&pm, 0, sizeof(pm));
             args.Npad = Npad;
-            static const int env_merge = [] { const char* e = getenv("DFW_TC_MERGE"); return e ? atoi(e) : 0; }();  // dev probe
-            args.nacc = env_merge ? 0 : 1;
-            static const int env_knock = [] { const char* e = getenv("DFW_TC_KNOCK"); return e ? atoi(e) : 0; }();  // dev probe: see Args::knock
-            args.knock = env_knock;
+            args.nacc = 1;
             int cols = 32;
             while (cols < 2 * regions * Npad) cols <<= 1;
             args.tmem_cols = cols;
@@ -1583,29 +1187,14 @@ int linear_tc_launch(const void* a1, const void* w1, int64_t k1, const void* a2,
     args.stages = stages;
     const size_t smem = carve(tf32, args.Npad, stages, out_boxes).total + 1024;
     const unsigned tiles = (unsigned)((args.N + kTileM - 1) / kTileM);
-    static const int env_cluster = [] { const char* e = getenv("DFW_TC_CLUSTER"); return e ? atoi(e) : 0; }();  // dev probe
-    unsigned cluster = env_cluster > 0 ? (unsigned)env_cluster : 1u;
-    if (tiles < 2 * cluster) cluster = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((tiles + cluster - 1) / cluster * cluster, 1, 1);
-    cfg.blockDim = dim3(kThreads, 1, 1);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cluster;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
     if (tf32) {
         auto kern = k_linear_tc<float, true>;
         DFW_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        DFW_CUDA(cudaLaunchKernelEx(&cfg, kern, maps, args));
+        kern<<<tiles, kThreads, smem, s>>>(maps, args);
     } else {
         auto kern = k_linear_tc<__nv_bfloat16, false>;
         DFW_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        DFW_CUDA(cudaLaunchKernelEx(&cfg, kern, maps, args));
+        kern<<<tiles, kThreads, smem, s>>>(maps, args);
     }
     DFW_LAUNCH_CHECK();
     return 0;

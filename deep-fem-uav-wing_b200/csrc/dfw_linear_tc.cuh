@@ -15,7 +15,6 @@ struct Args {
     int chunks[2];   // 128-byte K chunks per operand pair
     int stages;
     int flags;
-    int knock;       // dev probe (DFW_TC_KNOCK bit mask, persistent kernel only): 1 no conversion, 2 no MMA, 4 no weight loads, 8 no epilogue, 16 no activation loads
     const float* bias; const float* gamma; const float* beta; float eps;
     const float* row_scale;
     const void* residual; uint32_t drop_thr; float drop_scale; uint64_t seed;

@@ -50,28 +50,6 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, u
         "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
         : "memory");
 }
-// Same box delivered to the same shared-memory offset (and signalled on the same barrier offset) of every CTA of
-// the cluster named in `mask`: one L2 read feeds all of them.
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-            smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-        : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ uint32_t cluster_nctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {  // every thread of every CTA of the cluster
-    asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
 }
@@ -85,10 +63,6 @@ template <int CBYTES>
 __device__ __forceinline__ uint64_t make_desc_k(uint32_t saddr) {
     constexpr uint64_t sbo = CBYTES * 8, layout = CBYTES == 128 ? 2 : 4;
     return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)1 << 16) | ((sbo >> 4) << 32) | ((uint64_t)1 << 46) | (layout << 61);
-}
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
-    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)2 << 61);
 }
 
 template <bool TF32>
@@ -107,12 +81,6 @@ __device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t adesc, uint64_t b
 }
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// arrive on the barrier at this offset in every CTA of `mask` once the MMAs issued so far have retired
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-                 "h"(mask)
-                 : "memory");
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
     uint32_t r[32];
@@ -224,19 +192,6 @@ __device__ __forceinline__ uint32_t rna_tf32(float x) {
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
     return r;
 }
-
-
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* src, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(map)),
-                 "r"(smem_u32(src)), "r"(c0), "r"(c1)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void tma_store_wait_read() {
-    asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 128;" ::: "memory"); }  // the 4 epilogue warps only
 
 // One [128 rows x 128 B] box in SWIZZLE_128B layout: 16-byte chunk j of row r lives at r*128 + ((j ^ (r & 7)) << 4).
 // A thread that owns row r touches 8 distinct bank groups per quarter-warp: conflict-free.

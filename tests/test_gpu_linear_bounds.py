@@ -17,7 +17,7 @@ The 2u covers a tensor-core accumulation that truncates and the dropped lo*lo te
 WHICH kernel ran (torch.profiler kernel names), every raw-ABI output and workspace sits inside sentinel-filled guard bands,
 and every bf16 output of >= 1e5 elements is checked for a rounding bias (truncation instead of round-to-nearest-even).
 
-The kernel-selection switches (DFW_FORCE_SIMT, DFW_TC_PERSIST, DFW_TC_PAIR) are read once per process:
+The kernel-selection switches (DFW_FORCE_SIMT, DFW_TC_PERSIST) are read once per process:
 tests/test_gpu_linear_variants.py re-runs this file in a subprocess per switch, and the rows read os.environ to know
 which kernel to expect."""
 import json
@@ -48,7 +48,6 @@ def _atoi(s):
 # the same parsing as the library: force_simt() (dfw_linear.cu) and the atoi() switches of dfw_linear_tc.cu
 _simt_env = os.environ.get("DFW_FORCE_SIMT", "")
 SIMT = bool(_simt_env) and _simt_env[0] != "0"
-PAIR = _atoi(os.environ.get("DFW_TC_PAIR", "0")) != 0
 PERSIST = _atoi(os.environ.get("DFW_TC_PERSIST", "1")) != 0
 
 
@@ -313,25 +312,12 @@ def assert_kernels(row, names, expect, absent=()):
         assert not any(re.search(pat, n) for n in names), f"{row}: unexpected kernel matching {pat!r} in {sorted(set(names))}"
 
 
-def _pair_fits(tf32, npad, H, k1, k2):
-    """carve2() of dfw_linear_tc.cu: the CTA-pair kernel runs when its resident weight halves leave room for >= 3 stages."""
-    cb = 64 if tf32 else 128
-    e = 4 if tf32 else 2
-    chunks = -(-k1 * e // cb) + -(-k2 * e // cb)
-    w_lo = -(-(npad // 2) * cb // 1024) * 1024
-    stage = 128 * cb * (2 if tf32 else 1)
-    fixed = (2 * w_lo if tf32 else w_lo) * chunks + 8 * 2048 + 16 * (-(-H // 32) * 32) + 8 * (3 * 6 + 5) + 16
-    return fixed + 3 * stage + 1024 <= 227 * 1024
-
-
 def _tc_kernel(dtype, N, H, k1, k2):
     """The tensor-core forward kernel dfw_linear_fwd picks (dfw_linear_tc.cu, linear_tc_eligible / linear_tc_launch), or None."""
     e = 4 if dtype == F32 else 2
     if SIMT or not (16 <= H <= 256 and H % 16 == 0 and (H * e) % 128 == 0 and (k1 * e) % 16 == 0 and (k2 * e) % 16 == 0):
         return None
     npad, regions, tiles = (H + 15) // 16 * 16, 2 if dtype == F32 else 1, (N + 127) // 128
-    if PAIR and npad % 32 == 0 and 2 * regions * npad <= 512 and H % 32 == 0 and tiles >= 4 and _pair_fits(dtype == F32, npad, H, k1, k2):
-        return r"k_linear_tc2<"
     if PERSIST and 2 * regions * npad <= 512 and H % 32 == 0 and tiles >= 2:
         return r"k_linear_tcp<"
     return r"k_linear_tc<"
@@ -489,7 +475,7 @@ def test_linear_fwd_within_bounds(row, sign):
     keep = _keep(seed, N, H, p) if p else None
     ref = fwd_reference(a1, w1, a2, w2, bias, (gamma, beta) if ln else None, relu, keep, residual, rdw, rdb, dt == BF16)
     margins = _check_outputs(name, got, ref, dt == BF16)
-    record(f"linear_bounds/fwd/{name}/{sign}", kernel=sorted(set(names)), simt=SIMT, pair=PAIR, persist=PERSIST, **margins)
+    record(f"linear_bounds/fwd/{name}/{sign}", kernel=sorted(set(names)), simt=SIMT, persist=PERSIST, **margins)
 
 
 TINY_ROWS = [(k, h, dt) for k in (3, 10, 16) for h in (4, 64, 256) for dt in ("f32", "bf16", "f32_out_bf16")]

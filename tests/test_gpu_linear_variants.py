@@ -1,6 +1,6 @@
-"""The tensor-core linear has three kernels behind one entry point: the persistent one (default), the classic one-tile-per-CTA
-kernel (shapes the persistent kernel does not take; DFW_TC_PERSIST=0 forces it) and the opt-in CTA-pair kernel (DFW_TC_PAIR=1);
-DFW_FORCE_SIMT=1 sends every linear to the SIMT kernels.  The environment switches are read once per process, so the linear
+"""The tensor-core linear has two kernels behind one entry point: the persistent one (default) and the classic one-tile-per-CTA
+kernel (shapes the persistent kernel does not take; DFW_TC_PERSIST=0 forces it); DFW_FORCE_SIMT=1 sends every linear to the
+SIMT kernels.  The environment switches are read once per process, so the linear
 parity tests and the element-wise bounds of test_gpu_linear_bounds.py are re-run in a subprocess per variant."""
 import os
 import subprocess
@@ -12,7 +12,7 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [{"DFW_TC_PERSIST": "0"}, {"DFW_TC_PAIR": "1"}, {"DFW_FORCE_SIMT": "1"}], ids=["classic", "cta_pair", "simt"])
+@pytest.mark.parametrize("env", [{"DFW_TC_PERSIST": "0"}, {"DFW_FORCE_SIMT": "1"}], ids=["classic", "simt"])
 def test_linear_parity_suite_on_kernel_variant(env):
     e = dict(os.environ, **env)
     r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(REPO, "tests", "test_gpu_kernels.py"),

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Timing of the gather aggregation on the config-2 batch shapes (DFW_AGG_VARIANT is read once per process)."""
+"""Timing of the gather aggregation on the config-2 batch shapes."""
 import json, os, sys, torch
 REPO = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path[:0] = [REPO, os.path.join(REPO, "deep-fem-uav-wing_b200")]
@@ -14,7 +14,7 @@ def t(fn, iters=30):
         flush.zero_(); a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record(); fn(); b.record(); torch.cuda.synchronize(); ts.append(a.elapsed_time(b) * 1e3)
     ts.sort(); return round(ts[len(ts) // 2], 1)
-res = {"variant": os.environ.get("DFW_AGG_VARIANT", "0")}
+res = {}
 for kind in ("tri", "tet"):
     b = Batch.from_data_list([bench.to_data(m) for m in bench.make_meshes(range(4), kind)]).to("cuda")
     g = ops.get_graph(b.edge_index, b.x.shape[0]); rp_t, col_t = g.transpose()
