@@ -12,9 +12,13 @@
 // and a 16-bit slot per edge.  Per block the mean is then the dense product
 //        OUT[128, H] = ADJ[128, S] . X_staged[S, H]          (fp32 accumulation in TMEM, 1/deg applied in the epilogue)
 // with ADJ the block's 0/1 (multiplicity) matrix.  Every staged row crosses the L2 -> SM fabric and the LSU ONCE per block
-// (cp.async straight into the UMMA operand layout), the accumulation costs no SIMT instruction at all, and exactness is
-// kept: ADJ entries are small integers and the products of a bf16 row with them are exact, sums are fp32 (the result differs
-// from the CSR-order fp32 sum only by the association order: <= 1 bf16 ulp after the final rounding, tests/).
+// (cp.async straight into the UMMA operand layout) and the accumulation costs no SIMT instruction at all.  ADJ entries are
+// small integers and the products of a bf16 row with them are exact; the sums are fp32 in TMEM.  For finite inputs the result
+// differs from the CSR-order fp32 sum by the order and rounding of those additions only: before the final rounding, row i is
+// within (K_i 2^-23 + 2^-24) sum_j |s_i m_ij x_j| of the exact mean, K_i = 4 per 64-row chunk of its block (tc_agg_bound in
+// tests/test_gpu_aggregate_tc.py): relative to the sum of |terms|, so under cancellation more than one bf16 ulp of the result.
+// A non-finite row is different: the product multiplies every staged row by an ADJ column that is mostly zero (0 * Inf = NaN),
+// so a NaN or Inf source makes EVERY row of each block that stages it non-finite; the gather kernel poisons only its readers.
 //
 // One persistent CTA per SM, blocks taken in order blockIdx.x + i * gridDim.x (all SMs sweep the node array as one wavefront,
 // so neighbouring blocks' shared sources hit L2).  Warp roles, all decoupled by mbarriers:

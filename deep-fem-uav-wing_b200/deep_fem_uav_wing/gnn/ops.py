@@ -518,8 +518,10 @@ TC_AGG_MIN_REUSE = 3.0            # edges per staged row below which the gather 
 
 def aggregate_mean(graph: "CSRGraph", x):
     """Mean aggregation over ``graph``: the tensor-core block kernel when the graph carries a usable plan and the rows
-    qualify (bf16, H in 64/128/256), the gather kernel otherwise.  Both are deterministic; they differ by the association
-    order of fp32 additions only."""
+    qualify (bf16, H in 64/128/256), the gather kernel otherwise.  Both are deterministic.  For finite inputs they differ by
+    the order and rounding of the fp32 additions only (bounded relative to the sum of |terms|, not to the result: under
+    cancellation the bound allows more than one bf16 ulp of the result).  A NaN or Inf row poisons only the rows that read it in the gather kernel,
+    but every row of each 128-row block that stages it in the block kernel."""
     pl = graph.plan
     if pl is not None and pl.usable and pl.profitable and x.dtype == torch.bfloat16 and x.shape[1] in TC_AGG_WIDTHS:
         return aggregate_tc(pl, graph.inv_deg, x, graph.num_edges)

@@ -28,6 +28,8 @@ def c_oracle():
         lib.oracle_csr_build.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int] + [ctypes.c_void_p] * 4
         lib.oracle_csr_aggregate_f32.restype = None
         lib.oracle_csr_aggregate_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int64, ctypes.c_int64]
+        lib.oracle_csr_aggregate_ex_f32.restype = None
+        lib.oracle_csr_aggregate_ex_f32.argtypes = [ctypes.c_void_p] * 7 + [ctypes.c_int64, ctypes.c_int64]
         _LIB = lib
     return _LIB
 
@@ -55,4 +57,30 @@ def csr_aggregate_c(rowptr, col, inv_deg, x: np.ndarray) -> np.ndarray:
     c_oracle().oracle_csr_aggregate_f32(rowptr.ctypes.data, col.ctypes.data,
                                         inv_deg.ctypes.data if inv_deg is not None else None,
                                         x.ctypes.data, out.ctypes.data, x.shape[0], x.shape[1])
+    return out
+
+
+def csr_aggregate_ex(rowptr, col, x: np.ndarray, row_scale=None, src_scale=None, addend=None, n_rows=None) -> np.ndarray:
+    """The gather kernel's arithmetic in every form (``oracle_csr_aggregate_ex_f32``): per row, in CSR order,
+    ``acc = fmaf(x, src_scale[col], acc)`` or ``acc += x``, then ``fmaf(acc, row_scale, addend)`` or ``acc * row_scale``.
+    fp32 in, fp32 out; ``x`` may have more rows than the ``n_rows`` destination rows (default: as many)."""
+    def f32(a, shape):
+        if a is None:
+            return None
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        assert a.shape == shape, (a.shape, shape)
+        return a
+
+    x = np.ascontiguousarray(x, dtype=np.float32)
+    n = x.shape[0] if n_rows is None else int(n_rows)
+    H = x.shape[1]
+    rowptr = np.ascontiguousarray(rowptr, dtype=np.int32)
+    col = np.ascontiguousarray(col, dtype=np.int32)
+    assert rowptr.shape == (n + 1,) and int(rowptr[-1]) == col.size
+    assert col.size == 0 or (int(col.min()) >= 0 and int(col.max()) < x.shape[0])
+    row_scale, src_scale, addend = f32(row_scale, (n,)), f32(src_scale, (x.shape[0],)), f32(addend, (n, H))
+    out = np.empty((n, H), np.float32)
+    p = lambda a: None if a is None else a.ctypes.data
+    c_oracle().oracle_csr_aggregate_ex_f32(rowptr.ctypes.data, col.ctypes.data, p(row_scale), p(src_scale), x.ctypes.data,
+                                           p(addend), out.ctypes.data, n, H)
     return out

@@ -31,7 +31,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import record, rel_l2
+from helpers import Arena, assert_bound, assert_no_rounding_bias, bf16_ulp, launched_kernels, record, rel_l2, rounding_bias
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(REPO, "deep-fem-uav-wing_b200")
@@ -58,50 +58,6 @@ def short_bound(S, K, r=None, bf16=False):
     if bf16:
         b = b + 2.0 ** -8 * (r.double().abs() + b)
     return b
-
-
-def bound_margin(got, r, bound):
-    """(number of elements outside the bound, max |got - r| / bound).  An element with bound 0 must be exact; NaN fails."""
-    err = (got.double() - r.double()).abs()
-    bound = bound.double()
-    bad = ~(err <= bound)
-    ratio = torch.where(bound > 0, err / bound.clamp_min(1e-300), torch.where(err > 0, torch.inf, 0.0))
-    return int(bad.sum().item()), (float(ratio.max().item()) if ratio.numel() else 0.0)
-
-
-def assert_bound(name, got, r, bound):
-    nbad, margin = bound_margin(got, r, bound)
-    if nbad:
-        err = (got.double() - r.double()).abs() - bound.double()
-        i = int(torch.nan_to_num(err, nan=torch.inf).flatten().argmax())
-        g, rr, b = got.flatten()[i].item(), r.flatten()[i].item(), bound.flatten()[i].item()
-        raise AssertionError(f"{name}: {nbad} of {got.numel()} elements outside the bound (worst index {i}: got {g!r}, "
-                             f"exact {rr!r}, bound {b!r}, max err/bound {margin:.3g})")
-    return margin
-
-
-def bf16_ulp(r):
-    """One bf16 ulp at |r| (normal range)."""
-    a = r.double().abs().clamp_min(2.0 ** -126)
-    return torch.exp2(torch.floor(torch.log2(a)) - 7)
-
-
-def rounding_bias(got, r, pre_store_bound):
-    """Mean signed error of a bf16 store in ulps of r, signed toward |r| (a truncating store gives -0.5, RNE about 0),
-    over the elements whose pre-store error bound is below 1/8 ulp, where the rounding is what decides the error."""
-    r = r.double()
-    use = (r != 0) & (pre_store_bound.double() < 0.125 * bf16_ulp(r))
-    e = (got.double() - r) * torch.sign(r) / bf16_ulp(r)
-    return float(e[use].mean().item()) if bool(use.any()) else 0.0, int(use.sum().item())
-
-
-def assert_no_rounding_bias(name, got, r, pre_store_bound):
-    if got.numel() < 100_000:
-        return None
-    bias, n = rounding_bias(got, r, pre_store_bound)
-    assert n >= min(100_000, got.numel() // 2), f"{name}: only {n} elements qualify for the rounding-bias check"
-    assert abs(bias) < 0.05, f"{name}: mean signed bf16 store error {bias:+.4f} ulp over {n} elements (truncation gives -0.5)"
-    return bias
 
 
 def long_check(name, got, r, S, cpu32, extra=None, chain_bound=None):
@@ -260,48 +216,6 @@ def _seed(name):
     return zlib.crc32(name.encode()) & 0x7FFFFFFF
 
 
-class Arena:
-    """Device buffers inside sentinel-filled guard bands: check() asserts that no byte outside the handed-out ranges
-    changed.  The sentinel byte 0x7F reads as ~3.4e38 in fp32 and bf16, so an unwritten element fails its bound too."""
-
-    G = 4096
-    SENT = 0x7F
-
-    def __init__(self):
-        self.bufs = []
-
-    def out(self, shape, dtype, fill=None):
-        elt = torch.empty(0, dtype=dtype).element_size()
-        n = int(np.prod(shape)) * elt
-        raw = torch.full((n + 2 * self.G,), self.SENT, dtype=torch.uint8, device="cuda")
-        t = raw[self.G:self.G + n].view(dtype).view(shape)
-        if fill is not None:
-            t.copy_(fill)
-        self.bufs.append((raw, n))
-        return t
-
-    def ws(self, nbytes):
-        return self.out((int(nbytes),), torch.uint8), int(nbytes)
-
-    def check(self, name):
-        torch.cuda.synchronize()
-        for raw, n in self.bufs:
-            lo, hi = raw[:self.G], raw[self.G + n:]
-            assert bool((lo == self.SENT).all()) and bool((hi == self.SENT).all()), f"{name}: a byte outside an output or the workspace was written"
-
-
-def _launched(fn):
-    """Run fn() under torch.profiler and return (fn's result, names of the CUDA kernels it launched)."""
-    from torch.profiler import ProfilerActivity, profile
-
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        res = fn()
-        torch.cuda.synchronize()
-    names = [e.name for e in prof.events() if str(getattr(e, "device_type", "")).endswith("CUDA")]
-    return res, names
-
-
 def assert_kernels(row, names, expect, absent=()):
     if not names:
         print(f"[{row}] torch.profiler saw no CUDA kernels: the kernel-name assertion is skipped")
@@ -381,7 +295,7 @@ def _run_fwd(a1, w1, a2, w2, bias, gamma, beta, residual, p, seed, rdw, rdb, fla
                                            p, seed, _p(out), _p(pre), _p(stats), _p(rdw), _p(rdb), _p(rd), N, H, flags, _dt(a1),
                                            _p(ws), ws_bytes, _stream()))
 
-    _, names = _launched(call)
+    _, names = launched_kernels(call)
     return dict(out=out, pre=pre, stats=stats, rowdot=rd), names, ar
 
 
@@ -554,7 +468,7 @@ def test_linear_bwd_input_within_bounds(row, sign):
     ar = Arena()
     ga = ar.out((N, K), dt)
     ws, ws_bytes = ar.ws(cabi.lib.dfw_linear_ws_bytes(K, Hout, 0, _dt(g)))
-    _, names = _launched(lambda: cabi.check(cabi.lib.dfw_linear_bwd_input(g.data_ptr(), w.data_ptr(), rs.data_ptr(), add.data_ptr(), ga.data_ptr(),
+    _, names = launched_kernels(lambda: cabi.check(cabi.lib.dfw_linear_bwd_input(g.data_ptr(), w.data_ptr(), rs.data_ptr(), add.data_ptr(), ga.data_ptr(),
                                                                           N, Hout, K, _dt(g), ws.data_ptr(), ws_bytes, _stream())))
     ar.check(name)
     assert_kernels(name, names, _tc_kernel(dt, N, K, Hout, 0) or r"\bk_linear<")
@@ -676,7 +590,7 @@ def test_linear_bwd_weight_within_bounds(row, N):
                    "db": torch.randn(Hout, generator=gen, device="cuda") if want_db else None}
             outs = {k: (ar.out(v.shape, F32, fill=v if acc else None) if v is not None else None) for k, v in pre.items()}
             ws, _ = ar.ws(ws_bytes)
-            _, names = _launched(lambda: cabi.check(cabi.lib.dfw_linear_bwd_weight(
+            _, names = launched_kernels(lambda: cabi.check(cabi.lib.dfw_linear_bwd_weight(
                 _pn(g), _pn(a1), k1, _pn(a2), k2, outs["dw1"].data_ptr(), _p(outs["dw2"]), _p(outs["db"]), N, Hout, _dt(g), acc,
                 ws.data_ptr(), ws_bytes, _stream())))
             row_id = f"{name}/N{N}/{sign}/acc{acc}"
@@ -734,7 +648,7 @@ def _run_eb(g_out, g_rowdot, rdw, pre, stats, act, gamma, beta, p, seed, flags, 
     gy = ar.out((N, H), dt)
     o = {k: (ar.out((n,), F32) if k in want else None) for k, n in (("dgamma", H), ("dbeta", H), ("d_rowdot_w", H), ("d_rowdot_b", 1), ("d_bias", H))}
     ws, ws_bytes = ar.ws(cabi.lib.dfw_epilogue_bwd_ws_bytes(N, H))
-    _, names = _launched(lambda: cabi.check(cabi.lib.dfw_epilogue_bwd(
+    _, names = launched_kernels(lambda: cabi.check(cabi.lib.dfw_epilogue_bwd(
         _p(g_out), _p(g_rowdot), _p(rdw), _p(pre), _p(stats), _p(act), _p(gamma), _p(beta), p, seed, gy.data_ptr(), _p(o["dgamma"]),
         _p(o["dbeta"]), _p(o["d_rowdot_w"]), _p(o["d_rowdot_b"]), _p(o["d_bias"]), N, H, flags, int(dt == BF16),
         ws.data_ptr(), ws_bytes, _stream())))
