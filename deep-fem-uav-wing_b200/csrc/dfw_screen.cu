@@ -222,10 +222,39 @@ struct SummaryArgs {
     int log_scale;
 };
 
+// The screened-row rule of a case, shared by every per-case reduction over the model output: mask[row] != 0 when a mask
+// is given, else the root band pos_y > root_band * (max_y - min_y) of the row's own case (fem.py:637-640,
+// synth.py:154-155), from the per-chunk y ranges of k_chunk_minmax_y.  band_threshold is called by the whole block
+// (it synchronises); its scratch is a block-shared [kScrThreads / 32][2] float array.
+__device__ __forceinline__ double band_threshold(const float* __restrict__ mm, int64_t c0, int64_t c1, double root_band,
+                                                 float (*sh)[2], double* thr_s) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    float lo = FLT_MAX, hi = -FLT_MAX;
+    for (int64_t k = c0 + threadIdx.x; k < c1; k += blockDim.x) { lo = fminf(lo, mm[2 * k]); hi = fmaxf(hi, mm[2 * k + 1]); }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    if (lane == 0) { sh[wid][0] = lo; sh[wid][1] = hi; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < kScrThreads / 32; ++w) { lo = fminf(lo, sh[w][0]); hi = fmaxf(hi, sh[w][1]); }
+        *thr_s = root_band * ((double)hi - (double)lo);
+    }
+    __syncthreads();
+    return *thr_s;
+}
+
+__device__ __forceinline__ bool screened_row(const uint8_t* __restrict__ mask, const float* __restrict__ pos, int64_t i, double thr) {
+    return mask ? mask[i] != 0 : (double)pos[3 * i + 1] > thr;
+}
+
 template <typename T>
 __global__ void __launch_bounds__(kScrThreads) k_chunk_stats(const SummaryArgs p) {
     __shared__ double sh_sum[kScrThreads / 32];
     __shared__ float sh_f[kScrThreads / 32][4];
+    __shared__ float sh_band[kScrThreads / 32][2];
     __shared__ int64_t sh_arg[kScrThreads / 32];
     __shared__ int sh_n[kScrThreads / 32][4];
     __shared__ double thr_s;
@@ -237,23 +266,7 @@ __global__ void __launch_bounds__(kScrThreads) k_chunk_stats(const SummaryArgs p
         int64_t r0, r1;
         case_rows(p.case_ptr, b, p.N, r0, r1);
         const int64_t c0 = p.chunk_ptr[b], c1 = p.chunk_ptr[b + 1];
-        if (!p.mask) {  // root band of this case: pos_y > root_band * (max_y - min_y)  (fem.py:637-640, synth.py:154-155)
-            float lo = FLT_MAX, hi = -FLT_MAX;
-            for (int64_t k = c0 + threadIdx.x; k < c1; k += blockDim.x) { lo = fminf(lo, p.mm[2 * k]); hi = fmaxf(hi, p.mm[2 * k + 1]); }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
-                hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
-            }
-            if (lane == 0) { sh_f[wid][0] = lo; sh_f[wid][1] = hi; }
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                for (int w = 1; w < kScrThreads / 32; ++w) { lo = fminf(lo, sh_f[w][0]); hi = fmaxf(hi, sh_f[w][1]); }
-                thr_s = p.root_band * ((double)hi - (double)lo);
-            }
-            __syncthreads();
-        }
-        const double thr = p.mask ? 0.0 : thr_s;
+        const double thr = p.mask ? 0.0 : band_threshold(p.mm, c0, c1, p.root_band, sh_band, &thr_s);
         const int64_t beg = r0 + (c - c0) * kChunkRows, end = min(beg + kChunkRows, r1);
         double sum = 0.0;
         float mx = -INFINITY, mx_all = -INFINITY;
@@ -263,7 +276,7 @@ __global__ void __launch_bounds__(kScrThreads) k_chunk_stats(const SummaryArgs p
             float v = to_f32(pred[i]);
             if (p.log_scale) v = expm1f(v);  // inverse of log1p (dataset.py:148-151), as dfw_stress_metrics
             const bool fin = isfinite(v);
-            const bool scr = p.mask ? p.mask[i] != 0 : (double)p.pos[3 * i + 1] > thr;
+            const bool scr = screened_row(p.mask, p.pos, i, thr);
             n_bad += !fin;
             n_scr += scr;
             if (fin) {
@@ -365,6 +378,216 @@ SummaryWs carve_summary(void* ws, int64_t N, int64_t B) {
     return w;
 }
 
+// ---- per-case KS aggregate of the screened prediction and its seed gradient -------------------------------------------
+// Both reductions below reuse the summary's chunk plan and workspace: their per-chunk partials fit in its ChunkPart slots.
+struct KsPart {
+    double m;   // max of u over the chunk's set (after k_case_ks, in the case's first slot: over the case's set)
+    double s;   // sum over the set of exp(rho (u - m)); a row with u == m counts 1 (also when u = m = -inf)
+    int64_t n;  // rows in the set (0: m and s are meaningless)
+};
+static_assert(sizeof(KsPart) <= sizeof(ChunkPart) && alignof(KsPart) <= alignof(ChunkPart), "KS partials use the summary's slots");
+
+constexpr int kRowsPerThread = kChunkRows / kScrThreads;
+
+struct KsArgs {
+    const void* pred; const float* pos; const uint8_t* mask; const int64_t* case_ptr; const int64_t* chunk_ptr; const float* mm;
+    KsPart* part; float* seed;
+    int64_t B, N;
+    double root_band, rho;
+};
+
+__device__ __forceinline__ double ks_term(double rho, double u, double m) { return u == m ? 1.0 : exp(rho * (u - m)); }
+
+// the KS set S_b: screened rows whose fp32 stress expm1f(u) is finite - the rows behind max_stress_pa of the summary
+template <typename T>
+__device__ __forceinline__ void ks_load(const KsArgs& p, int64_t beg, int64_t end, double thr, float (&u)[kRowsPerThread],
+                                        bool (&in)[kRowsPerThread]) {
+    const T* __restrict__ pred = static_cast<const T*>(p.pred);
+#pragma unroll
+    for (int k = 0; k < kRowsPerThread; ++k) {
+        const int64_t i = beg + threadIdx.x + (int64_t)k * kScrThreads;
+        u[k] = 0.f;
+        in[k] = false;
+        if (i < end) {
+            u[k] = to_f32(pred[i]);
+            in[k] = isfinite(expm1f(u[k])) && screened_row(p.mask, p.pos, i, thr);
+        }
+    }
+}
+
+// per chunk: its max m and sum exp(rho (u - m)) in fp64; rows in ascending order per thread, lanes by a fixed butterfly,
+// warps in index order
+template <typename T>
+__global__ void __launch_bounds__(kScrThreads) k_chunk_ks(const KsArgs p) {
+    __shared__ float sh_band[kScrThreads / 32][2];
+    __shared__ float sh_m[kScrThreads / 32];
+    __shared__ int sh_n[kScrThreads / 32];
+    __shared__ double sh_s[kScrThreads / 32];
+    __shared__ double thr_s;
+    __shared__ float m_s;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int64_t total = p.chunk_ptr[p.B];
+    for (int64_t c = blockIdx.x; c < total; c += gridDim.x) {
+        const int64_t b = chunk_case(p.chunk_ptr, p.B, c);
+        int64_t r0, r1;
+        case_rows(p.case_ptr, b, p.N, r0, r1);
+        const int64_t c0 = p.chunk_ptr[b], c1 = p.chunk_ptr[b + 1];
+        const double thr = p.mask ? 0.0 : band_threshold(p.mm, c0, c1, p.root_band, sh_band, &thr_s);
+        const int64_t beg = r0 + (c - c0) * kChunkRows, end = min(beg + kChunkRows, r1);
+        float u[kRowsPerThread];
+        bool in[kRowsPerThread];
+        ks_load<T>(p, beg, end, thr, u, in);
+        float mx = -INFINITY;
+        int n = 0;
+#pragma unroll
+        for (int k = 0; k < kRowsPerThread; ++k) {
+            if (in[k]) { mx = fmaxf(mx, u[k]); ++n; }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+            n += __shfl_xor_sync(0xffffffffu, n, o);
+        }
+        if (lane == 0) { sh_m[wid] = mx; sh_n[wid] = n; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < kScrThreads / 32; ++w) { mx = fmaxf(mx, sh_m[w]); n += sh_n[w]; }
+            m_s = mx;
+        }
+        __syncthreads();
+        const double m = (double)m_s;
+        double s = 0.0;
+#pragma unroll
+        for (int k = 0; k < kRowsPerThread; ++k) {
+            if (in[k]) s += ks_term(p.rho, (double)u[k], m);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (lane == 0) sh_s[wid] = s;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < kScrThreads / 32; ++w) s += sh_s[w];
+            KsPart q;
+            q.m = m; q.s = s; q.n = n;
+            p.part[c] = q;
+        }
+        __syncthreads();
+    }
+}
+
+// one thread per case: its chunks in ascending order, each rescaled to the running max; the case's (m, s, n) goes back
+// into its first chunk slot for k_chunk_ks_seed.  out[b] = [KS_b = m + ln(s) / rho, n]; [0, 0] for an empty set.
+__global__ void k_case_ks(const int64_t* __restrict__ chunk_ptr, KsPart* __restrict__ part, int64_t B, double rho,
+                          double* __restrict__ out) {
+    for (int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; b < B; b += (int64_t)gridDim.x * blockDim.x) {
+        double m = -INFINITY, s = 0.0;
+        int64_t n = 0;
+        const int64_t c0 = chunk_ptr[b], c1 = chunk_ptr[b + 1];
+        for (int64_t c = c0; c < c1; ++c) {
+            const KsPart q = part[c];
+            if (q.n == 0) continue;
+            if (n == 0) {
+                m = q.m; s = q.s;
+            } else if (q.m > m) {
+                s = s * ks_term(rho, m, q.m) + q.s;
+                m = q.m;
+            } else {
+                s += q.s * ks_term(rho, q.m, m);
+            }
+            n += q.n;
+        }
+        out[2 * b] = n ? m + log(s) / rho : 0.0;
+        out[2 * b + 1] = (double)n;
+        if (c0 < c1) {
+            KsPart q;
+            q.m = m; q.s = s; q.n = n;
+            part[c0] = q;
+        }
+    }
+}
+
+// one write per row: w = exp(rho (u - m_b)) / s_b on S_b, computed in fp64 and rounded to fp32 once; 0 elsewhere
+template <typename T>
+__global__ void __launch_bounds__(kScrThreads) k_chunk_ks_seed(const KsArgs p) {
+    __shared__ float sh_band[kScrThreads / 32][2];
+    __shared__ double thr_s;
+    const int64_t total = p.chunk_ptr[p.B];
+    for (int64_t c = blockIdx.x; c < total; c += gridDim.x) {
+        const int64_t b = chunk_case(p.chunk_ptr, p.B, c);
+        int64_t r0, r1;
+        case_rows(p.case_ptr, b, p.N, r0, r1);
+        const int64_t c0 = p.chunk_ptr[b], c1 = p.chunk_ptr[b + 1];
+        const double thr = p.mask ? 0.0 : band_threshold(p.mm, c0, c1, p.root_band, sh_band, &thr_s);
+        const int64_t beg = r0 + (c - c0) * kChunkRows, end = min(beg + kChunkRows, r1);
+        const KsPart q = p.part[c0];
+        float u[kRowsPerThread];
+        bool in[kRowsPerThread];
+        ks_load<T>(p, beg, end, thr, u, in);
+#pragma unroll
+        for (int k = 0; k < kRowsPerThread; ++k) {
+            const int64_t i = beg + threadIdx.x + (int64_t)k * kScrThreads;
+            if (i < end) p.seed[i] = (in[k] && q.n > 0) ? __double2float_rn(ks_term(p.rho, (double)u[k], q.m) / q.s) : 0.f;
+        }
+    }
+}
+
+// ---- per-case column sums ----------------------------------------------------------------------------------------------
+constexpr int kColGroup = (int)(sizeof(ChunkPart) / sizeof(double));  // columns per pass: one ChunkPart slot of doubles
+
+// per chunk: fp64 sums of columns [col0, col0 + ng) of a fp32 [N, C]; same fixed order as k_chunk_ks
+__global__ void __launch_bounds__(kScrThreads) k_chunk_colsum(const float* __restrict__ a, int64_t C, int64_t col0, int ng,
+                                                               const int64_t* __restrict__ case_ptr, const int64_t* __restrict__ chunk_ptr,
+                                                               int64_t B, int64_t N, double* __restrict__ part /*[chunks][kColGroup]*/) {
+    __shared__ double sh[kScrThreads / 32][kColGroup];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int64_t total = chunk_ptr[B];
+    for (int64_t c = blockIdx.x; c < total; c += gridDim.x) {
+        const int64_t b = chunk_case(chunk_ptr, B, c);
+        int64_t r0, r1;
+        case_rows(case_ptr, b, N, r0, r1);
+        const int64_t beg = r0 + (c - chunk_ptr[b]) * kChunkRows, end = min(beg + kChunkRows, r1);
+        double acc[kColGroup];
+#pragma unroll
+        for (int j = 0; j < kColGroup; ++j) acc[j] = 0.0;
+        for (int64_t i = beg + threadIdx.x; i < end; i += blockDim.x) {
+            const float* __restrict__ row = a + i * C + col0;
+#pragma unroll
+            for (int j = 0; j < kColGroup; ++j)
+                if (j < ng) acc[j] += (double)row[j];
+        }
+#pragma unroll
+        for (int j = 0; j < kColGroup; ++j) {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], o);
+        }
+        if (lane == 0) {
+#pragma unroll
+            for (int j = 0; j < kColGroup; ++j) sh[wid][j] = acc[j];
+        }
+        __syncthreads();
+        if (threadIdx.x < ng) {  // one thread per column, warps in index order
+            const int j = threadIdx.x;
+            double t = sh[0][j];
+            for (int w = 1; w < kScrThreads / 32; ++w) t += sh[w][j];
+            part[c * kColGroup + j] = t;
+        }
+        __syncthreads();
+    }
+}
+
+// one thread per (case, column): the case's chunks in ascending order
+__global__ void k_case_colsum(const int64_t* __restrict__ chunk_ptr, const double* __restrict__ part, int64_t B, int ng,
+                              int64_t nc, int64_t j0, double* __restrict__ out) {
+    const int64_t total = B * ng;
+    for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = t / ng;
+        const int j = (int)(t % ng);
+        double sum = 0.0;
+        for (int64_t c = chunk_ptr[b]; c < chunk_ptr[b + 1]; ++c) sum += part[c * kColGroup + j];
+        out[b * nc + j0 + j] = sum;
+    }
+}
+
 }  // namespace
 }  // namespace dfw
 
@@ -438,5 +661,76 @@ extern "C" int dfw_case_stress_summary(const void* pred, int dtype, const float*
     const int fgrid = (int)std::max<int64_t>(1, std::min<int64_t>((B + 127) / 128, (int64_t)kNumSMs * 4));
     k_case_finalize<<<fgrid, 128, 0, s>>>(case_ptr, w.chunk_ptr, w.part, B, N, out);
     DFW_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int dfw_case_ks_seed(const void* pred, int dtype, const float* pos, const uint8_t* mask, const int64_t* case_ptr, int64_t B,
+                                int64_t N, double root_band, double rho, double* out, float* seed, void* ws, size_t ws_bytes,
+                                dfw_stream_t stream) {
+    using namespace dfw;
+    DFW_REQUIRE(dtype == DFW_F32 || dtype == DFW_BF16, "dfw_case_ks_seed: unknown dtype %d", dtype);
+    DFW_REQUIRE(B >= 0 && N >= 0, "dfw_case_ks_seed: negative size (B=%lld, N=%lld)", (long long)B, (long long)N);
+    DFW_REQUIRE(rho > 0.0 && rho < INFINITY, "dfw_case_ks_seed: rho must be positive and finite (got %g)", rho);
+    if (B == 0) return 0;
+    DFW_REQUIRE(case_ptr && out, "dfw_case_ks_seed: null case_ptr or output");
+    DFW_REQUIRE(N == 0 || (pred && seed && (pos || mask)), "dfw_case_ks_seed: null pred, seed or pos");
+    SummaryWs w = carve_summary(ws, N, B);
+    DFW_REQUIRE(ws && ws_bytes >= w.bytes, "dfw_case_ks_seed: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const int64_t mc = max_chunks(N, B);
+    k_chunk_scan<<<1, kScanBlock, 0, s>>>(case_ptr, B, N, mc, w.chunk_ptr);
+    DFW_LAUNCH_CHECK();
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(mc, (int64_t)kNumSMs * 8));
+    if (!mask) {
+        k_chunk_minmax_y<<<grid, kScrThreads, 0, s>>>(pos, case_ptr, w.chunk_ptr, B, N, w.mm);
+        DFW_LAUNCH_CHECK();
+    }
+    KsArgs a{};
+    a.pred = pred; a.pos = pos; a.mask = mask; a.case_ptr = case_ptr; a.chunk_ptr = w.chunk_ptr; a.mm = w.mm;
+    a.part = reinterpret_cast<KsPart*>(w.part); a.seed = seed;
+    a.B = B; a.N = N; a.root_band = root_band; a.rho = rho;
+    if (dtype == DFW_F32)
+        k_chunk_ks<float><<<grid, kScrThreads, 0, s>>>(a);
+    else
+        k_chunk_ks<__nv_bfloat16><<<grid, kScrThreads, 0, s>>>(a);
+    DFW_LAUNCH_CHECK();
+    const int fgrid = (int)std::max<int64_t>(1, std::min<int64_t>((B + 127) / 128, (int64_t)kNumSMs * 4));
+    k_case_ks<<<fgrid, 128, 0, s>>>(w.chunk_ptr, a.part, B, rho, out);
+    DFW_LAUNCH_CHECK();
+    if (dtype == DFW_F32)
+        k_chunk_ks_seed<float><<<grid, kScrThreads, 0, s>>>(a);
+    else
+        k_chunk_ks_seed<__nv_bfloat16><<<grid, kScrThreads, 0, s>>>(a);
+    DFW_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int dfw_case_column_sums(const float* a, int64_t N, int64_t C, int64_t c0, int64_t nc, const int64_t* case_ptr, int64_t B,
+                                    double* out, void* ws, size_t ws_bytes, dfw_stream_t stream) {
+    using namespace dfw;
+    DFW_REQUIRE(N >= 0 && C >= 0 && c0 >= 0 && nc >= 0 && B >= 0,
+                "dfw_case_column_sums: negative size (N=%lld, C=%lld, c0=%lld, nc=%lld, B=%lld)", (long long)N, (long long)C,
+                (long long)c0, (long long)nc, (long long)B);
+    DFW_REQUIRE(c0 + nc <= C, "dfw_case_column_sums: columns [%lld, %lld) outside the %lld columns of a", (long long)c0,
+                (long long)(c0 + nc), (long long)C);
+    if (B == 0 || nc == 0) return 0;
+    DFW_REQUIRE(case_ptr && out, "dfw_case_column_sums: null case_ptr or output");
+    DFW_REQUIRE(N == 0 || a, "dfw_case_column_sums: null input");
+    SummaryWs w = carve_summary(ws, N, B);
+    DFW_REQUIRE(ws && ws_bytes >= w.bytes, "dfw_case_column_sums: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const int64_t mc = max_chunks(N, B);
+    k_chunk_scan<<<1, kScanBlock, 0, s>>>(case_ptr, B, N, mc, w.chunk_ptr);
+    DFW_LAUNCH_CHECK();
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(mc, (int64_t)kNumSMs * 8));
+    double* part = reinterpret_cast<double*>(w.part);
+    for (int64_t j0 = 0; j0 < nc; j0 += kColGroup) {  // the chunk slots hold kColGroup columns: one pass per group
+        const int ng = (int)std::min<int64_t>(kColGroup, nc - j0);
+        k_chunk_colsum<<<grid, kScrThreads, 0, s>>>(a, C, c0 + j0, ng, case_ptr, w.chunk_ptr, B, N, part);
+        DFW_LAUNCH_CHECK();
+        const int fgrid = (int)std::max<int64_t>(1, std::min<int64_t>((B * ng + 127) / 128, (int64_t)kNumSMs * 4));
+        k_case_colsum<<<fgrid, 128, 0, s>>>(w.chunk_ptr, part, B, ng, nc, j0, out);
+        DFW_LAUNCH_CHECK();
+    }
     return 0;
 }

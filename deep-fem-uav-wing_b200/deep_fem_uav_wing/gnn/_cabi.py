@@ -88,6 +88,10 @@ SIGNATURES = {
     "dfw_case_stress_summary_ws_bytes": (c_size_t, [c_int64, c_int64]),
     "dfw_case_stress_summary": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_double, c_double, c_int,
                                         c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dfw_case_ks_seed": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_double, c_double, c_void_p,
+                                 c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dfw_case_column_sums": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_size_t,
+                                     c_void_p]),
     "dfw_cast": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_void_p]),
 }
 

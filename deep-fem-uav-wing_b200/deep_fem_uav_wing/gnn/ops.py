@@ -684,16 +684,18 @@ def linear_fwd(a1, w1, a2=None, w2=None, bias=None, ln=None, eps=1e-5, relu=Fals
 
 
 def epilogue_bwd(g_out, N, Hout, dtype_like, *, g_rowdot=None, rowdot_w=None, pre=None, stats=None, act=None, ln=None,
-                 relu=False, dropout_p=0.0, seed=0, want_bias_grad=False):
+                 relu=False, dropout_p=0.0, seed=0, want_bias_grad=False, want_param_grads=True):
+    """``dfw_epilogue_bwd``.  ``want_param_grads=False``: the LayerNorm affine and row-dot parameter gradients come back as
+    None and, with ``want_bias_grad=False``, the kernel skips its column pass (only ``g_y`` is computed)."""
     dev = dtype_like.device
     seed_v, seed_flag = _seed_arg(seed)
     flags = (EP_RELU if relu else 0) | (EP_LAYERNORM if ln is not None else 0) | ((EP_DROPOUT | seed_flag) if dropout_p > 0.0 else 0)
     g_y = torch.empty(N, Hout, dtype=dtype_like.dtype, device=dev)
     dgamma = dbeta = d_rw = d_rb = None
-    if ln is not None:
+    if ln is not None and want_param_grads:
         dgamma = torch.empty(Hout, dtype=torch.float32, device=dev)
         dbeta = torch.empty(Hout, dtype=torch.float32, device=dev)
-    if g_rowdot is not None:
+    if g_rowdot is not None and want_param_grads:
         d_rw = torch.empty(Hout, dtype=torch.float32, device=dev)
         d_rb = torch.empty(1, dtype=torch.float32, device=dev)
     d_bias = torch.empty(Hout, dtype=torch.float32, device=dev) if want_bias_grad else None
@@ -707,7 +709,7 @@ def epilogue_bwd(g_out, N, Hout, dtype_like, *, g_rowdot=None, rowdot_w=None, pr
             _ptr(ln[0]) if ln is not None else None, _ptr(ln[1]) if ln is not None else None, float(dropout_p),
             seed_v, g_y.data_ptr(), _ptr(dgamma), _ptr(dbeta), _ptr(d_rw), _ptr(d_rb), _ptr(d_bias), N, Hout, flags,
             _DTYPES[dtype_like.dtype], ws.data_ptr(), ws_bytes, _stream(dtype_like)))
-    LAUNCH_COUNTER["kernels"] += 2 if (ln is not None or g_rowdot is not None or want_bias_grad) else 1
+    LAUNCH_COUNTER["kernels"] += 2 if (dgamma is not None or d_rw is not None or want_bias_grad) else 1
     return g_y, dgamma, dbeta, d_rw, d_rb, d_bias
 
 
@@ -791,13 +793,18 @@ def vertex_normals(pos: torch.Tensor, faces: torch.Tensor):
     return normal, status
 
 
-def case_stress_summary(pred, pos, case_ptr, mask=None, root_band: float = 0.05, allowable_pa: float | None = None,
-                        log_scale: bool = True) -> torch.Tensor:
-    """``dfw_case_stress_summary``: float64 [B,8] on the device, one record per case of ``case_ptr`` (int64 [B+1], device):
-    [rows, screened rows, max stress, its row within the case (-1: none), mean stress, max stress over all rows,
-    screened rows above ``allowable_pa``, non-finite stresses].  Screened rows are ``mask`` (uint8/bool [N]) or, without
-    it, ``pos_y > root_band * (max_y - min_y)`` of the case.  ``pred`` [N] or [N,1], fp32 or bf16, ``log1p(stress)`` when
-    ``log_scale``.  Deterministic and independent of how cases are batched; no host synchronisation."""
+def _case_ptr_arg(case_ptr: torch.Tensor, device, what: str) -> tuple[torch.Tensor, int]:
+    if case_ptr.dtype != torch.int64 or case_ptr.device != device:
+        raise TypeError(f"case_ptr must be an int64 tensor on the device of {what}")
+    cp = case_ptr.contiguous()
+    B = int(cp.numel()) - 1
+    if B < 0:
+        raise ValueError("case_ptr needs at least one entry")
+    return cp, B
+
+
+def _case_inputs(pred, pos, case_ptr, mask):
+    """Checked, contiguous arguments of the per-case reductions over the model output: (pred, pos, case_ptr, mask, N, B)."""
     _require_cuda(pred, "pred")
     p = pred.detach().contiguous()
     N = int(p.shape[0]) if p.dim() > 0 else 1
@@ -806,18 +813,24 @@ def case_stress_summary(pred, pos, case_ptr, mask=None, root_band: float = 0.05,
     pos = pos.to(torch.float32).contiguous()
     if tuple(pos.shape) != (N, 3):
         raise ValueError(f"pos must be [{N}, 3], got {tuple(pos.shape)}")
-    if case_ptr.dtype != torch.int64 or case_ptr.device != p.device:
-        raise TypeError("case_ptr must be an int64 tensor on the device of pred")
-    cp = case_ptr.contiguous()
-    B = int(cp.numel()) - 1
-    if B < 0:
-        raise ValueError("case_ptr needs at least one entry")
+    cp, B = _case_ptr_arg(case_ptr, p.device, "pred")
     m = None
     if mask is not None:
         m = mask.detach().reshape(-1).contiguous()
         m = m.view(torch.uint8) if m.dtype == torch.bool else m.to(torch.uint8)
         if m.numel() != N:
             raise ValueError(f"mask has {m.numel()} entries for {N} rows")
+    return p, pos, cp, m, N, B
+
+
+def case_stress_summary(pred, pos, case_ptr, mask=None, root_band: float = 0.05, allowable_pa: float | None = None,
+                        log_scale: bool = True) -> torch.Tensor:
+    """``dfw_case_stress_summary``: float64 [B,8] on the device, one record per case of ``case_ptr`` (int64 [B+1], device):
+    [rows, screened rows, max stress, its row within the case (-1: none), mean stress, max stress over all rows,
+    screened rows above ``allowable_pa``, non-finite stresses].  Screened rows are ``mask`` (uint8/bool [N]) or, without
+    it, ``pos_y > root_band * (max_y - min_y)`` of the case.  ``pred`` [N] or [N,1], fp32 or bf16, ``log1p(stress)`` when
+    ``log_scale``.  Deterministic and independent of how cases are batched; no host synchronisation."""
+    p, pos, cp, m, N, B = _case_inputs(pred, pos, case_ptr, mask)
     out = torch.empty(max(B, 0), 8, dtype=torch.float64, device=p.device)
     ws_bytes = lib.dfw_case_stress_summary_ws_bytes(N, B)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=p.device)
@@ -826,6 +839,48 @@ def case_stress_summary(pred, pos, case_ptr, mask=None, root_band: float = 0.05,
         check(lib.dfw_case_stress_summary(p.data_ptr(), _dt(p), pos.data_ptr(), _ptr(m), cp.data_ptr(), B, N, float(root_band), allow,
                                           int(bool(log_scale)), out.data_ptr(), ws.data_ptr(), ws_bytes, _stream(p)))
     LAUNCH_COUNTER["kernels"] += (3 if m is not None else 4) if B > 0 else 0
+    return out
+
+
+def case_ks_seed(pred, pos, case_ptr, mask=None, root_band: float = 0.05, rho: float = 100.0):
+    """``dfw_case_ks_seed``: a smooth per-case peak of ``pred`` (log1p of the stress) and its gradient, on the device.
+
+    Per case b, S_b is the set ``case_stress_summary`` takes ``max_stress_pa`` over (screened rows - ``mask`` or the root
+    band - whose fp32 stress is finite).  With ``m_b = max u`` and ``s_b = sum exp(rho (u - m_b))`` over S_b, returns
+    float64 [B,2] ``[KS_b = m_b + ln(s_b) / rho, |S_b|]`` (``[0, 0]`` for an empty set) and the seed fp32 [N]
+    ``w = exp(rho (u - m_b)) / s_b`` on S_b, 0 elsewhere (``dKS_b / du``).  ``max u <= KS_b <= max u + ln|S_b| / rho``.
+    Deterministic and independent of how cases are batched; no host synchronisation."""
+    if not rho > 0.0 or rho == float("inf"):
+        raise ValueError(f"rho must be positive and finite, got {rho}")
+    p, pos, cp, m, N, B = _case_inputs(pred, pos, case_ptr, mask)
+    out = torch.empty(max(B, 0), 2, dtype=torch.float64, device=p.device)
+    seed = torch.empty(N, dtype=torch.float32, device=p.device)
+    ws_bytes = lib.dfw_case_stress_summary_ws_bytes(N, B)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=p.device)
+    with torch.cuda.device(p.device), _prof("case_ks_seed", N * (2 * _esz(p) + 2 * (12 if m is None else 1) + 4) + 8 * (B + 1) + 16 * B):
+        check(lib.dfw_case_ks_seed(p.data_ptr(), _dt(p), pos.data_ptr(), _ptr(m), cp.data_ptr(), B, N, float(root_band), float(rho),
+                                   out.data_ptr(), seed.data_ptr(), ws.data_ptr(), ws_bytes, _stream(p)))
+    LAUNCH_COUNTER["kernels"] += (4 if m is not None else 5) if B > 0 else 0
+    return out, seed
+
+
+def case_column_sums(a, case_ptr, c0: int, nc: int) -> torch.Tensor:
+    """``dfw_case_column_sums``: float64 [B,nc], the sums over each case's rows of columns ``c0 .. c0+nc-1`` of the fp32 [N,C]
+    ``a`` (fp64, fixed order: independent of how cases are batched).  The screener passes the input gradient with
+    ``c0 = 6, nc = 4``."""
+    _require_cuda(a, "a")
+    if a.dtype != torch.float32 or a.dim() != 2:
+        raise TypeError(f"case_column_sums takes a float32 [N, C] tensor, got {a.dtype} {tuple(a.shape)}")
+    a = a.detach().contiguous()
+    N, C = int(a.shape[0]), int(a.shape[1])
+    cp, B = _case_ptr_arg(case_ptr, a.device, "a")
+    out = torch.empty(max(B, 0), int(nc), dtype=torch.float64, device=a.device)
+    ws_bytes = lib.dfw_case_stress_summary_ws_bytes(N, B)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=a.device)
+    with torch.cuda.device(a.device), _prof("case_column_sums", 4 * N * C + 8 * (B + 1) + 8 * B * int(nc)):
+        check(lib.dfw_case_column_sums(a.data_ptr(), N, C, int(c0), int(nc), cp.data_ptr(), B, out.data_ptr(), ws.data_ptr(), ws_bytes,
+                                       _stream(a)))
+    LAUNCH_COUNTER["kernels"] += 1 + 2 * ((int(nc) + 4) // 5) if (B > 0 and nc > 0) else 0
     return out
 
 
@@ -1114,18 +1169,22 @@ class SageConvFn(_Fn):
         graph: CSRGraph = ctx.graph
         g_out = g_out.contiguous()
         N, H = g_out.shape
-        dgamma = dbeta = dbl = None
+        # no parameter gradient wanted (design sensitivities: only the input gradient): no weight-gradient work at all
+        want_params = any(ctx.needs_input_grad[1:6])
+        dgamma = dbeta = dbl = dwl = dwr = None
         if ctx.fused_tail:
             # the epilogue backward also emits the column sums of g_y = lin_l's bias gradient
             g_y, dgamma, dbeta, _, _, dbl = epilogue_bwd(g_out, N, H, g_out, pre=pre, stats=stats, ln=(gamma, beta), relu=True,
-                                                         dropout_p=ctx.dropout_p, seed=ctx.seed, want_bias_grad=ctx.has_bias)
+                                                         dropout_p=ctx.dropout_p, seed=ctx.seed,
+                                                         want_bias_grad=ctx.has_bias and want_params, want_param_grads=want_params)
         else:
             g_y = g_out
-        fork = _fork_dw(g_y, ctx.needs_input_grad[0])
-        with fork:
-            dwl, dwr, db_ = linear_bwd_weight(g_y, agg, x, want_bias=ctx.has_bias and not ctx.fused_tail)
-        if not ctx.fused_tail:
-            dbl = db_
+        fork = _fork_dw(g_y, ctx.needs_input_grad[0] and want_params)
+        if want_params:
+            with fork:
+                dwl, dwr, db_ = linear_bwd_weight(g_y, agg, x, want_bias=ctx.has_bias and not ctx.fused_tail)
+            if not ctx.fused_tail:
+                dbl = db_
         g_x = None
         if ctx.needs_input_grad[0]:
             # dL/dx = A^T D^-1 (g_y W_l) + g_y W_r (+ g_out) = (A^T D^-1 g_y) W_l + g_y W_r (+ g_out): aggregate the
@@ -1161,19 +1220,22 @@ class LinearFn(_Fn):
         x, wc, act = ctx.saved_tensors
         g_out = g_out.contiguous()
         N, H = g_out.shape
+        want_params = any(ctx.needs_input_grad[1:3])
+        dw = None
         if ctx.relu or ctx.dropout_p > 0.0:
             if H % 4 != 0:
                 raise RuntimeError("dfw_b200: ReLU/dropout backward needs out_features % 4 == 0")
             g_y, _, _, _, _, db = epilogue_bwd(g_out, N, H, g_out, act=act, relu=ctx.relu, dropout_p=ctx.dropout_p, seed=ctx.seed,
-                                               want_bias_grad=ctx.has_bias)
+                                               want_bias_grad=ctx.has_bias and want_params)
             want_db = False
         else:
             g_y, db, want_db = g_out, None, ctx.has_bias
-        fork = _fork_dw(g_y, ctx.needs_input_grad[0])
-        with fork:
-            dw, _, db_ = linear_bwd_weight(g_y, x, None, want_bias=want_db)
-        if want_db:
-            db = db_
+        fork = _fork_dw(g_y, ctx.needs_input_grad[0] and want_params)
+        if want_params:
+            with fork:
+                dw, _, db_ = linear_bwd_weight(g_y, x, None, want_bias=want_db)
+            if want_db:
+                db = db_
         g_x = linear_bwd_input(g_y, wc) if ctx.needs_input_grad[0] else None
         fork.join()
         return g_x, dw, db, None, None, None
@@ -1209,14 +1271,19 @@ class DecoderTailFn(_Fn):
         N = h.shape[0]
         Hmid = hid.shape[1]
         g_r = g_out.reshape(-1).float().contiguous()
+        want_params = any(ctx.needs_input_grad[1:5])
         g_y, _, _, dw4, db4, db3 = epilogue_bwd(None, N, Hmid, hid, g_rowdot=g_r, rowdot_w=w4f, act=hid, relu=True,
-                                                dropout_p=ctx.dropout_p, seed=ctx.seed, want_bias_grad=ctx.has_b3)
-        fork = _fork_dw(g_y, ctx.needs_input_grad[0])
-        with fork:
-            dw3, _, _ = linear_bwd_weight(g_y, h, None, want_bias=False)
+                                                dropout_p=ctx.dropout_p, seed=ctx.seed, want_bias_grad=ctx.has_b3 and want_params,
+                                                want_param_grads=want_params)
+        fork = _fork_dw(g_y, ctx.needs_input_grad[0] and want_params)
+        dw3 = None
+        if want_params:
+            with fork:
+                dw3, _, _ = linear_bwd_weight(g_y, h, None, want_bias=False)
         g_h = linear_bwd_input(g_y, w3c) if ctx.needs_input_grad[0] else None
         fork.join()
-        return g_h, dw3, db3, dw4.reshape(1, -1), (db4 if ctx.has_b4 else None), None, None
+        return (g_h, dw3, db3, dw4.reshape(1, -1) if dw4 is not None else None, (db4 if ctx.has_b4 and want_params else None),
+                None, None)
 
 
 class MaskedMSEFn(torch.autograd.Function):

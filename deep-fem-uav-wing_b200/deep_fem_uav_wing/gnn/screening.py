@@ -16,6 +16,31 @@ them into launches of up to ``max_nodes_per_launch`` nodes and per launch runs, 
 The host waits for the device only when the pinned result ring wraps and after the last launch, so the enqueue of
 launch l+1 overlaps the GPU work of launch l.  Every kernel on the path is row-local with a fixed per-row order, so a
 case's result does not depend on which cases share its launch.
+
+Design sensitivities (``sensitivities=True``): which way to move a design to lower its peak stress.  Per case b, S_b is
+the set ``max_stress_pa`` is taken over (screened rows with a finite prediction) and ``u = pred`` (log1p of the stress):
+
+    m_b = max u,  s_b = sum exp(rho (u - m_b)),  KS_b = m_b + ln(s_b) / rho        (over S_b;  rho = ks_rho)
+    ks_stress_pa = expm1(KS_b),   max_stress_pa <= ks_stress_pa <= expm1(log1p(max_stress_pa) + ln|S_b| / rho)
+
+a smooth upper bound of the peak stress, and its gradient with respect to the four wing parameters.  These enter the
+model only through ``x[:, 6:10] = global_params(...)`` (reference ``dataset.py:122-127``), so with ``g_x`` the gradient of
+``sum_b KS_b`` with respect to ``x`` (the cases of a launch are a disjoint union: one backward serves them all)
+
+    d ks_stress_pa / d span_m = exp(KS_b) * sum over the rows of case b of g_x[:, 6] / 1.0
+
+and likewise ``chord_m`` (column 7, / 0.3), ``sweep_deg`` (8, / 30) and ``thickness_ratio`` (9, / 0.10): Pa/m, Pa/m,
+Pa/deg and Pa per unit thickness ratio.  This is the surrogate's PARTIAL derivative with the mesh held fixed - positions
+and normals unchanged.  (Positions are min-max normalised per axis, so a mesh stretched along one axis keeps its
+normalised positions, but its normals change; gradients with respect to node positions are not computed.)  Per launch,
+after the summary: the forward runs under grad mode with ``x`` tracked and the parameters not,
+
+    dfw_case_ks_seed                    [B,2] (KS_b, |S_b|) and the seed dKS_b/du [N]
+    torch.autograd.grad(pred, x, seed)  the model's input-gradient backward; no weight-gradient kernel runs
+    dfw_case_column_sums(g_x, 6, 4)     [B,4] -> with the summary, one [B,14] record per case, one D2H copy
+
+still without a host wait per launch.  ``rho`` trades smoothness for tightness: the bound above is reached when every
+row of S_b has the peak value, and a case whose peak stands out sits near ``max_stress_pa``.
 """
 from __future__ import annotations
 
@@ -77,6 +102,20 @@ def global_params(params: dict) -> np.ndarray:
                      (params["thickness_ratio"] - 0.05) / 0.10], dtype=np.float32)
 
 
+PARAM_SCALE = {"span_m": 1.0, "chord_m": 0.3, "sweep_deg": 30.0, "thickness_ratio": 0.10}  # the divisors of global_params
+
+
+def sensitivity_record(r: np.ndarray) -> dict:
+    """``ks_stress_pa`` and ``d_ks_stress_pa`` from the device record ``[KS_b, |S_b|, sum g_x[:, 6:10] over the case]``:
+    ``d expm1(KS) / dp = exp(KS) * dKS/dx_col / scale``, in fp64.  None for both when S_b is empty."""
+    ks, n = float(r[0]), int(r[1])
+    if n == 0:
+        return {"ks_stress_pa": None, "d_ks_stress_pa": None}
+    f = np.exp(np.float64(ks))
+    return {"ks_stress_pa": float(np.expm1(np.float64(ks))),
+            "d_ks_stress_pa": {k: float(f * np.float64(r[2 + j]) / s) for j, (k, s) in enumerate(PARAM_SCALE.items())}}
+
+
 class _Case:
     __slots__ = ("case_id", "node_id", "pos", "pos32", "normal", "rows", "skipped", "gp", "error")
 
@@ -112,20 +151,30 @@ class DesignScreener:
     ``max_stress_node_id`` and ``max_stress_pos`` (the case's own id and units), ``mean_stress_pa``,
     ``max_stress_all_nodes_pa`` and, with ``allowable_pa``, ``n_over_allowable`` and
     ``margin_of_safety = allowable / max - 1``.  A case whose prediction is not finite is ``"failed"``.
-    fp32 or bf16 follows the model's ``set_compute_dtype``."""
+    fp32 or bf16 follows the model's ``set_compute_dtype``.
+
+    ``sensitivities=True`` adds ``ks_stress_pa`` (the KS bound of the peak stress with ``rho = ks_rho``, see the module
+    docstring) and ``d_ks_stress_pa = {"span_m", "chord_m", "sweep_deg", "thickness_ratio"}``, its partial derivatives
+    with the mesh held fixed (Pa/m, Pa/m, Pa/deg, Pa per unit thickness ratio); both are None for a case with no screened
+    row.  Every other field is the same, bit for bit, as without sensitivities.  The caller's model is not modified:
+    no parameter gets a ``.grad`` and ``requires_grad`` is left as it is."""
 
     def __init__(self, model, max_nodes_per_launch: int = 320_000, root_band: float = 0.05, allowable_pa: float | None = None,
-                 result_ring: int = 8, prep_threads: int = 4):
+                 result_ring: int = 8, prep_threads: int = 4, sensitivities: bool = False, ks_rho: float = 100.0):
         if int(getattr(model, "out_channels", 1)) != 1:
             raise ValueError("DesignScreener needs a model with out_channels = 1 (one stress value per node)")
         if allowable_pa is not None and not allowable_pa > 0:
             raise ValueError("allowable_pa must be positive")
+        if not (0.0 < ks_rho < float("inf")):
+            raise ValueError("ks_rho must be positive and finite")
         self.model = model
         self.max_nodes = int(max_nodes_per_launch)
         self.root_band = float(root_band)
         self.allowable_pa = None if allowable_pa is None else float(allowable_pa)
         self.result_ring = max(1, int(result_ring))
         self.prep_threads = max(1, int(prep_threads))
+        self.sensitivities = bool(sensitivities)
+        self.ks_rho = float(ks_rho)
         self.device = next(model.parameters()).device
         if self.device.type != "cuda":
             raise RuntimeError("DesignScreener: the model must live on a CUDA device (deep_fem_uav_wing.gnn has no CPU fallback)")
@@ -191,10 +240,23 @@ class DesignScreener:
                         normal[ptr[b]:ptr[b + 1]].copy_(launch["normal"][ptr[b]:ptr[b + 1]])
         x, _ = ops.node_features_batched(pos, normal, None, launch["gp"], cp, launch["max_rows"])
         graph, _ = ops.faces_to_graph(faces, launch["N"], want_edge_index=False, sync=False)
-        with torch.no_grad():
-            pred = self.model(x, graph)  # eval + no_grad + CSRGraph: the one-call dfw_graphsage_forward
+        if self.sensitivities:
+            # grad mode with x tracked and the parameters detached: the piecewise forward (bit-identical to the one-call
+            # path) saves what the input-gradient backward needs, and no weight-gradient kernel runs
+            params = {k: v.detach() for k, v in self.model.named_parameters()}
+            x.requires_grad_()
+            with torch.enable_grad():
+                pred = torch.func.functional_call(self.model, params, (x, graph))
+        else:
+            with torch.no_grad():
+                pred = self.model(x, graph)  # eval + no_grad + CSRGraph: the one-call dfw_graphsage_forward
         summary = ops.case_stress_summary(pred, pos, cp, None, self.root_band, self.allowable_pa, log_scale=True)
-        res = torch.empty(launch["B"], 8, dtype=torch.float64, pin_memory=True)
+        if self.sensitivities:
+            ks, seed = ops.case_ks_seed(pred, pos, cp, None, self.root_band, self.ks_rho)
+            g_x, = torch.autograd.grad(pred, x, seed.view_as(pred))
+            dks = ops.case_column_sums(g_x, cp, 6, 4)
+            summary = torch.cat([summary, ks, dks], dim=1)
+        res = torch.empty(launch["B"], summary.shape[1], dtype=torch.float64, pin_memory=True)
         res.copy_(summary, non_blocking=True)
         launch["result"] = res
         launch["done"] = torch.cuda.Event()
@@ -231,6 +293,8 @@ class DesignScreener:
         if self.allowable_pa is not None:
             d["n_over_allowable"] = int(r[6])
             d["margin_of_safety"] = self.allowable_pa / float(r[2]) - 1.0 if r[2] > 0 else None
+        if self.sensitivities:
+            d.update(sensitivity_record(r[8:]))
         return d
 
     def _prepare(self, cases: Iterable[dict]) -> Iterator[_Case]:

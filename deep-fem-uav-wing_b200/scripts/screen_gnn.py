@@ -4,6 +4,8 @@
 Cases come from geometry packs (``--cases-dir``, written by ``caseio.pack_geometry_case``), from the dataset's FEM case
 files (``--all`` over ``data/raw``: their normals are used, their stress is not) or are generated (``--synthetic N``).
 One JSON line per case goes to ``--out`` in input order, and the ``--top-k`` designs by peak stress are printed.
+``--sensitivities`` adds to every line the KS bound of the peak stress (``ks_stress_pa``, ``--ks-rho``) and its partial
+derivatives with respect to span, chord, sweep and thickness ratio with the mesh held fixed (``d_ks_stress_pa``).
 With ``torchrun`` the case list is sharded ``case_ids[rank::world]`` as in ``inference_gnn.py``; the data path has no
 communication, and at the end a gloo group gathers the records to rank 0, which writes the one output file.
 """
@@ -62,6 +64,9 @@ def main():
     p.add_argument("--root-band", type=float, default=0.05)
     p.add_argument("--max-nodes-per-launch", type=int, default=320_000)
     p.add_argument("--top-k", type=int, default=10)
+    p.add_argument("--sensitivities", action="store_true",
+                   help="add ks_stress_pa and its gradient d_ks_stress_pa with respect to the four wing parameters")
+    p.add_argument("--ks-rho", type=float, default=100.0, help="KS aggregation parameter of --sensitivities (larger: closer to the max)")
     p.add_argument("--out", type=str, default="screening.jsonl", help="JSON lines, one per case in input order (relative to --root)")
     args = p.parse_args()
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -79,7 +84,8 @@ def main():
     if args.dtype == "bf16":
         model.set_compute_dtype(torch.bfloat16)
     allowable = args.allowable_mpa * 1e6 if args.allowable_mpa is not None else None
-    screener = DesignScreener(model, max_nodes_per_launch=args.max_nodes_per_launch, root_band=args.root_band, allowable_pa=allowable)
+    screener = DesignScreener(model, max_nodes_per_launch=args.max_nodes_per_launch, root_band=args.root_band, allowable_pa=allowable,
+                              sensitivities=args.sensitivities, ks_rho=args.ks_rho)
     cases = case_list(args, root)
     mine = list(range(len(cases)))[rank::world]
 

@@ -343,6 +343,29 @@ int dfw_case_stress_summary(const void* pred, int dtype, const float* pos, const
                             int64_t B, int64_t N, double root_band, double allowable_pa, int log_scale, double* out,
                             void* ws, size_t ws_bytes, dfw_stream_t stream);
 
+/* (s3) Design sensitivities: a smooth per-case peak of the model output and its seed gradient.  Per case b, S_b is the
+ *     set behind max stress in (s2): screened rows (the same mask / root-band rule) whose fp32 stress expm1f(u) is finite,
+ *     u = pred (log1p of the stress).  With m_b = max over S_b of u and s_b = sum over S_b of exp(rho (u - m_b)):
+ *         out float64 [B,2] = [KS_b = m_b + ln(s_b) / rho, |S_b|]        ([0, 0] when S_b is empty)
+ *         seed fp32 [N]     = exp(rho (u - m_b)) / s_b on S_b, 0 on every other row of a case    (= dKS_b / du)
+ *     so max u <= KS_b <= max u + ln|S_b| / rho.  A row with u == m_b counts exp(0) = 1 (also when both are -inf).
+ *     rho > 0 and finite.  Rows outside [case_ptr[0], case_ptr[B]) are not written.  pos may be NULL when mask is given.
+ *     Chunk plan of (s2): per chunk the max and the fp64 sum of exp(rho (u - m_chunk)) in a fixed order, chunks combined in
+ *     ascending order with the usual rescaling; the seed of a row is computed in fp64 and rounded to fp32 once.  A case's
+ *     record and seed depend on its own rows only, bitwise.  No float atomics, no host synchronisation.
+ *     ws: dfw_case_stress_summary_ws_bytes(N, B) bytes (the same chunk plan; no query of its own).
+ *
+ * (s4) Per-case column sums: out float64 [B,nc] = sum over the rows of case b of a[row, c0 + j], j < nc, for a fp32 [N,C]
+ *     (the screener passes the input gradient g_x [N,10] with c0 = 6, nc = 4: the gradient with respect to the four scaled
+ *     wing parameters).  fp64 sums over 2048-row chunks counted from the case's first row, chunks in ascending order: a
+ *     record depends on its own case only, bitwise.  ws: dfw_case_stress_summary_ws_bytes(N, B) bytes.
+ * ---------------------------------------------------------------------------------------- */
+int dfw_case_ks_seed(const void* pred, int dtype, const float* pos, const uint8_t* mask, const int64_t* case_ptr, int64_t B,
+                     int64_t N, double root_band, double rho, double* out, float* seed, void* ws, size_t ws_bytes,
+                     dfw_stream_t stream);
+int dfw_case_column_sums(const float* a, int64_t N, int64_t C, int64_t c0, int64_t nc, const int64_t* case_ptr, int64_t B,
+                         double* out, void* ws, size_t ws_bytes, dfw_stream_t stream);
+
 /* dtype conversion helper (weights fp32 -> bf16 copies for the bf16 path) */
 int dfw_cast(const void* src, int src_dtype, void* dst, int dst_dtype, int64_t n, dfw_stream_t stream);
 
