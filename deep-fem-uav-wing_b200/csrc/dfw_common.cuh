@@ -85,6 +85,20 @@ __device__ __forceinline__ float from_f32<float>(float x) { return x; }
 template <>
 __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
 
+// min / max that return NaN when either operand is NaN, as numpy's minimum / maximum do (fminf / fmaxf return the
+// other operand, so a reduction built on them drops a NaN).  The float forms are one PTX instruction (sm_80+).
+__device__ __forceinline__ float min_nan(float a, float b) {
+    float r;
+    asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
+__device__ __forceinline__ float max_nan(float a, float b) {
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
+__device__ __forceinline__ double max_nan(double a, double b) { return (a > b || a != a) ? a : b; }
+
 // Counter-based dropout RNG: the keep-mask is a pure function of (seed, row, column), so the backward regenerates
 // it instead of storing a mask.  Two levels, both the 32-bit "lowbias32" finaliser: a key per ROW (computed once by
 // the thread or warp that owns the row) and ~9 integer instructions per element.  (The first version hashed a

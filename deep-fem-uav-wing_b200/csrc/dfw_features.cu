@@ -5,10 +5,11 @@
 //   y = log1p(stress_vm)                                                                [N,1]  fp32
 // with the reference's guards (range < 1e-8 -> 1, dataset.py:135; |normal| < 1e-8 -> 1, dataset.py:140).
 // The arithmetic is written with the non-contracting intrinsics (__fmul_rn / __fadd_rn / __fsqrt_rn / __fdiv_rn) in
-// numpy's evaluation order, so x is BIT-IDENTICAL to the reference's float32 result; y uses log1pf, which may differ
-// from numpy's float32 log1p in the last ulp (tests allow 2 ulp).
+// numpy's evaluation order, so x is BIT-IDENTICAL to the reference's float32 result (a zero may differ in sign: numpy's
+// min over +0 and -0 depends on their order); y uses log1pf, within 1 ulp of the correctly rounded log1p.
 // Two launches: a per-axis min/max reduction (fixed order: min/max are exact whatever the order) and one
-// element-wise pass.  HBM-bound; algorithmic bytes = 28 N read + 44 N written.
+// element-wise pass.  The min/max propagate NaN as numpy's pos.min(axis=0) does: a NaN coordinate makes that axis of
+// its case NaN in every row.  HBM-bound; algorithmic bytes = 28 N read + 44 N written.
 #include <algorithm>
 #include <cfloat>
 
@@ -30,16 +31,16 @@ __global__ void __launch_bounds__(kFeatThreads) k_pos_minmax(const float* __rest
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
             const float v = pos[3 * i + a];
-            lo[a] = fminf(lo[a], v);
-            hi[a] = fmaxf(hi[a], v);
+            lo[a] = min_nan(lo[a], v);
+            hi[a] = max_nan(hi[a], v);
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
-            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
+            lo[a] = min_nan(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
+            hi[a] = max_nan(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
         }
     }
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -51,7 +52,7 @@ __global__ void __launch_bounds__(kFeatThreads) k_pos_minmax(const float* __rest
     if (threadIdx.x < 6) {
         const int k = threadIdx.x;
         float v = sh[0][k];
-        for (int w = 1; w < kFeatThreads / 32; ++w) v = k < 3 ? fminf(v, sh[w][k]) : fmaxf(v, sh[w][k]);
+        for (int w = 1; w < kFeatThreads / 32; ++w) v = k < 3 ? min_nan(v, sh[w][k]) : max_nan(v, sh[w][k]);
         part[6 * (int64_t)blockIdx.x + k] = v;
     }
     __syncthreads();
@@ -64,7 +65,7 @@ __global__ void __launch_bounds__(kFeatThreads) k_pos_minmax(const float* __rest
         __threadfence();
         const int k = threadIdx.x;
         float v = part[k];
-        for (unsigned b = 1; b < gridDim.x; ++b) v = k < 3 ? fminf(v, part[6 * (int64_t)b + k]) : fmaxf(v, part[6 * (int64_t)b + k]);
+        for (unsigned b = 1; b < gridDim.x; ++b) v = k < 3 ? min_nan(v, part[6 * (int64_t)b + k]) : max_nan(v, part[6 * (int64_t)b + k]);
         mm[k] = v;
         if (k == 0) *ticket = 0u;
     }
@@ -125,16 +126,16 @@ __global__ void __launch_bounds__(kFeatThreads) k_pos_minmax_cases(const float* 
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
             const float v = pos[3 * i + a];
-            lo[a] = fminf(lo[a], v);
-            hi[a] = fmaxf(hi[a], v);
+            lo[a] = min_nan(lo[a], v);
+            hi[a] = max_nan(hi[a], v);
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
-            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
+            lo[a] = min_nan(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
+            hi[a] = max_nan(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
         }
     }
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -146,7 +147,7 @@ __global__ void __launch_bounds__(kFeatThreads) k_pos_minmax_cases(const float* 
     if (threadIdx.x < 6) {
         const int k = threadIdx.x;
         float v = sh[0][k];
-        for (int w = 1; w < kFeatThreads / 32; ++w) v = k < 3 ? fminf(v, sh[w][k]) : fmaxf(v, sh[w][k]);
+        for (int w = 1; w < kFeatThreads / 32; ++w) v = k < 3 ? min_nan(v, sh[w][k]) : max_nan(v, sh[w][k]);
         mm[8 * (int64_t)blockIdx.x + k] = v;
     }
 }

@@ -5,7 +5,8 @@
 // there, pred / target / mask are copied to the host in full (model.py:173-179), expm1'd (model.py:184-185) and
 // reduced once per subset (model.py:190-204), once per validation batch (scripts/train_gnn.py:85-107).  Here one
 // kernel reads the three arrays once and leaves 8 doubles on the device; the caller copies 64 bytes.
-// Deterministic: fixed grid, fixed-order second pass, no float atomics.
+// Deterministic: fixed grid, fixed-order second pass, no float atomics.  Every max stage propagates NaN, so a NaN
+// error makes mae, rmse and max_error of its subset NaN alike, as numpy does.
 // Roofline: HBM, algorithmic bytes = N*C*2*b + N (mask); a 200k-node batch is launch-latency bound.
 #include <algorithm>
 
@@ -40,9 +41,9 @@ __global__ void __launch_bounds__(kMetThreads) k_stress_metrics(const T* __restr
             t = expm1f(t);
         }
         const float e = fabsf(p - t);
-        sa[0] += e; sq[0] = fmaf(e, e, sq[0]); mx[0] = fmaxf(mx[0], e); cn[0] += 1.f;
+        sa[0] += e; sq[0] = fmaf(e, e, sq[0]); mx[0] = max_nan(mx[0], e); cn[0] += 1.f;
         if (mask && mask[i / C]) {
-            sa[1] += e; sq[1] = fmaf(e, e, sq[1]); mx[1] = fmaxf(mx[1], e); cn[1] += 1.f;
+            sa[1] += e; sq[1] = fmaf(e, e, sq[1]); mx[1] = max_nan(mx[1], e); cn[1] += 1.f;
         }
     }
     double v[8] = {(double)sa[0], (double)sq[0], (double)mx[0], (double)cn[0], (double)sa[1], (double)sq[1], (double)mx[1], (double)cn[1]};
@@ -51,7 +52,7 @@ __global__ void __launch_bounds__(kMetThreads) k_stress_metrics(const T* __restr
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
             const double w = __shfl_xor_sync(0xffffffffu, v[k], o);
-            v[k] = (k == 2 || k == 6) ? fmax(v[k], w) : v[k] + w;
+            v[k] = (k == 2 || k == 6) ? max_nan(v[k], w) : v[k] + w;
         }
     }
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -63,7 +64,7 @@ __global__ void __launch_bounds__(kMetThreads) k_stress_metrics(const T* __restr
     if (threadIdx.x == 0) {
         double a[8] = {0, 0, 0, 0, 0, 0, 0, 0};
         for (int w = 0; w < kMetThreads / 32; ++w)
-            for (int k = 0; k < 8; ++k) a[k] = (k == 2 || k == 6) ? fmax(a[k], sh[w][k]) : a[k] + sh[w][k];
+            for (int k = 0; k < 8; ++k) a[k] = (k == 2 || k == 6) ? max_nan(a[k], sh[w][k]) : a[k] + sh[w][k];
         for (int k = 0; k < 8; ++k) part[8 * (int64_t)blockIdx.x + k] = a[k];
         __threadfence();
         last = atomicAdd(ticket, 1u) == gridDim.x - 1;
@@ -75,7 +76,7 @@ __global__ void __launch_bounds__(kMetThreads) k_stress_metrics(const T* __restr
         double a = 0.0;
         for (unsigned b = 0; b < gridDim.x; ++b) {
             const double w = part[8 * (int64_t)b + k];
-            a = (k == 2 || k == 6) ? fmax(a, w) : a + w;
+            a = (k == 2 || k == 6) ? max_nan(a, w) : a + w;
         }
         sh[0][k] = a;
     }

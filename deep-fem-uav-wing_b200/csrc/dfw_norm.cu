@@ -534,8 +534,9 @@ extern "C" int dfw_masked_mse_bwd(const void* pred, const void* target, const ui
                                   dfw_stream_t stream) {
     using namespace dfw;
     DFW_REQUIRE(dtype == DFW_F32 || dtype == DFW_BF16, "dfw_masked_mse_bwd: unknown dtype %d", dtype);
-    DFW_REQUIRE(N >= 0 && C >= 1 && result && g_loss && g_pred, "dfw_masked_mse_bwd: bad arguments");
-    if (N == 0) return 0;
+    DFW_REQUIRE(N >= 0 && C >= 1 && result && g_loss, "dfw_masked_mse_bwd: bad arguments");
+    if (N == 0) return 0;  // an empty gradient has no storage: its pointer is null
+    DFW_REQUIRE(g_pred, "dfw_masked_mse_bwd: null g_pred");
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const int64_t total = N * C;
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((total + 255) / 256, (int64_t)kNumSMs * 8));

@@ -747,10 +747,14 @@ def linear_bwd_weight(g_y, a1, a2=None, want_bias=True):
 
 def stress_metrics(pred, target, mask=None, log_scale=True) -> torch.Tensor:
     """``dfw_stress_metrics``: 8 doubles on the device - [mae, rmse, max_error, count] for all nodes, then for the
-    masked nodes (``compute_metrics``, reference ``model.py:156-216``).  No host synchronisation."""
+    masked nodes (``compute_metrics``, reference ``model.py:156-216``).  No host synchronisation.  When the dtypes of
+    ``pred`` and ``target`` differ, both are read in fp32: rounding an fp32 target to bf16 before ``expm1`` would cost up
+    to 2^-8 relative in log space."""
     _require_cuda(pred, "pred")
-    p = pred.detach().contiguous()
-    t = target.detach().to(p.dtype).contiguous()
+    p, t = pred.detach(), target.detach()
+    if p.dtype != t.dtype:
+        p, t = p.float(), t.float()
+    p, t = p.contiguous(), t.contiguous()
     N = p.shape[0] if p.dim() > 0 else 1
     C = p.numel() // max(N, 1) if N > 0 else 1
     m = None

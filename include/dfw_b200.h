@@ -97,7 +97,9 @@ int dfw_faces_to_csr(const int64_t* faces, int64_t F, const int64_t* sorted_ids,
 /* Node features of build_graph_data (dataset.py:129-151) on the device:
  *   x [N,10] fp32 = [(pos - min)/range | normal/|normal| | global_params4], y [N,1] fp32 = log1p(stress) (nullable).
  *   pos, normal fp32 [N,3], stress fp32 [N] on the device; global_params4 = 4 HOST floats (dataset.py:122-127).
- *   x is bit-identical to the reference's numpy float32 arithmetic; y may differ in the last ulp (log1pf). */
+ *   x is bit-identical to the reference's numpy float32 arithmetic, NaN included: a NaN coordinate makes that axis's
+ *   min/max, and so column a of every row of the case, NaN, as numpy's pos.min(axis=0) does (a zero may differ in sign,
+ *   numpy's min over +0 and -0 depends on their order).  y is within 1 ulp of the correctly rounded log1p (log1pf). */
 size_t dfw_node_features_ws_bytes(int64_t N);
 int dfw_node_features(const float* pos, const float* normal, const float* stress, const float* global_params4,
                       int normalize_pos, int log_scale, float* x, float* y, int64_t N, void* ws, size_t ws_bytes,
@@ -298,7 +300,9 @@ int dfw_masked_mse_bwd(const void* pred, const void* target, const uint8_t* mask
  * D2H copies of model.py:173-179.  result (device, 8 doubles) =
  *   [mae, rmse, max_error, count] over all N*C elements, then the same over rows with mask[row] != 0;
  * log_scale != 0 applies expm1 to pred and target first (model.py:184-185); an empty subset reports zeros
- * (model.py:194-195); mask == NULL makes both halves equal (model.py:207-210).  Deterministic.
+ * (model.py:194-195); mask == NULL makes both halves equal (model.py:207-210).  With C > 1, mask[i / C] selects
+ * element i (the mask is per row).  A NaN error makes mae, rmse and max_error of its subset NaN, as numpy does.
+ * pred and target share dtype.  Deterministic.
  * ---------------------------------------------------------------------------------------- */
 size_t dfw_stress_metrics_ws_bytes(int64_t N, int64_t C);
 int dfw_stress_metrics(const void* pred, const void* target, const uint8_t* mask, int64_t N, int64_t C,
