@@ -48,6 +48,9 @@ extern "C" int dfw_sage_layer_fwd(const int32_t* rowptr, const int32_t* col, con
     DFW_REQUIRE(!(flags & DFW_EP_RESIDUAL) || Hin == Hout, "dfw_sage_layer_fwd: the residual h + h_new needs Hin == Hout (%lld, %lld)",
                 (long long)Hin, (long long)Hout);
     DFW_REQUIRE(!(flags & DFW_EP_TRANSPOSE_W), "dfw_sage_layer_fwd: weights are [Hout, Hin]");
+    // dfw_linear_fwd takes a short workspace as "no tensor cores": the one-call layer would silently change kernels (and bits)
+    const size_t need = dfw_sage_layer_fwd_ws_bytes(N, Hin, Hout, dtype);
+    DFW_REQUIRE(ws_bytes >= need && (ws || need == 0), "dfw_sage_layer_fwd: workspace too small (%zu < %zu)", ws_bytes, need);
     int rc = dfw_sage_aggregate(rowptr, col, inv_deg, x, nullptr, agg, N, E, Hin, dtype, stream);
     if (rc) return rc;
     return dfw_linear_fwd(agg, w_l, Hin, x, w_r, Hin, b_l, ln_gamma, ln_beta, ln_eps, (flags & DFW_EP_RESIDUAL) ? x : nullptr, dropout_p,
@@ -155,6 +158,8 @@ extern "C" int dfw_mlp2_fwd(const void* x, const void* w1, const float* b1, cons
     using namespace dfw;
     DFW_REQUIRE(mode == DFW_MLP2_ENCODER || mode == DFW_MLP2_DECODER, "dfw_mlp2_fwd: unknown mode %d", mode);
     DFW_REQUIRE(x && w1 && w2 && out, "dfw_mlp2_fwd: null pointer");
+    const size_t need = dfw_mlp2_fwd_ws_bytes(N, K, Hmid, Hout, dtype);  // see dfw_sage_layer_fwd
+    DFW_REQUIRE(ws_bytes >= need && (ws || need == 0), "dfw_mlp2_fwd: workspace too small (%zu < %zu)", ws_bytes, need);
     const int seed_flag = flags & DFW_EP_SEED_IS_PTR;
     if (mode == DFW_MLP2_ENCODER) {
         DFW_REQUIRE(hidden, "dfw_mlp2_fwd: the encoder needs the hidden buffer");

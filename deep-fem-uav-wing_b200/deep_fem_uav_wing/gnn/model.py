@@ -219,6 +219,9 @@ class MaskedMSELoss(nn.Module):
     sync.  With an all-False mask the value is 0 as in the reference; the reference returns a
     fresh leaf there (no gradient reaches the model), here the gradient is exactly zero.  Pass
     ``strict_empty=True`` to reproduce the fresh-leaf behaviour (costs one host sync).
+
+    As ``F.mse_loss``: a bf16 prediction against an fp32 target (a model fed bf16 features) is
+    computed in fp32 from the unrounded target, and its gradient comes back in bf16.
     """
 
     def __init__(self, reduction: str = "mean", strict_empty: bool = False):

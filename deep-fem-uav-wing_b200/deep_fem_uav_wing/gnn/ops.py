@@ -1291,11 +1291,17 @@ class DecoderTailFn(_Fn):
 
 
 class MaskedMSEFn(torch.autograd.Function):
+    """When the dtypes of ``pred`` and ``target`` differ, both are read in fp32 (the upcast is exact; rounding an fp32
+    target to bf16 would move the difference by up to 2^-9 |target|) and the fp32 gradient is rounded once to ``pred``'s
+    dtype.  Equal dtypes are computed in that dtype."""
+
     @staticmethod
     def forward(ctx, pred, target, mask, reduction_mean):
         _require_cuda(pred, "pred")
         pred_c = pred.contiguous()
-        target_c = target.to(pred.dtype).contiguous()
+        target_c = target.contiguous()
+        if pred_c.dtype != target_c.dtype:
+            pred_c, target_c = _f32(pred_c), _f32(target_c)
         N = pred_c.shape[0]
         C = pred_c.numel() // max(N, 1) if N > 0 else 1
         m = None
@@ -1313,7 +1319,7 @@ class MaskedMSEFn(torch.autograd.Function):
         LAUNCH_COUNTER["kernels"] += 1
         ctx.save_for_backward(pred_c, target_c, m, result)
         ctx.reduction_mean = reduction_mean
-        ctx.shape = pred.shape
+        ctx.shape, ctx.pred_dtype = pred.shape, pred.dtype
         loss, count = result[0], result[1]
         ctx.mark_non_differentiable(count)
         return loss, count
@@ -1329,4 +1335,4 @@ class MaskedMSEFn(torch.autograd.Function):
             check(lib.dfw_masked_mse_bwd(pred_c.data_ptr(), target_c.data_ptr(), _ptr(m), result.data_ptr(), gl.data_ptr(), N, C,
                                          int(ctx.reduction_mean), _dt(pred_c), g.data_ptr(), _stream(pred_c)))
         LAUNCH_COUNTER["kernels"] += 1
-        return g.view(ctx.shape), None, None, None
+        return cast(g, ctx.pred_dtype).view(ctx.shape), None, None, None

@@ -286,6 +286,9 @@ int dfw_mlp2_bwd(const void* x, const void* hidden, const void* out, const void*
  *   result fp32 [2]: [0] = loss (mean: sum/max(count,1); sum: sum), [1] = number of selected
  *   elements.  mask uint8 [N] (nullable = all rows).  pred/target fp32 or bf16 [N,C].
  *   bwd: g_pred = g_loss * 2 (pred-target) * mask / (mean ? max(count,1) : 1).
+ *   pred and target share dtype.  MaskedMSELoss (gnn/ops.py:MaskedMSEFn) calls the fp32 entry
+ *   when they differ (a bf16 prediction against an fp32 target): both are read in fp32, the loss
+ *   is fp32 and the fp32 gradient is rounded once to pred's dtype.
  * ---------------------------------------------------------------------------------------- */
 size_t dfw_masked_mse_ws_bytes(int64_t N, int64_t C);
 int dfw_masked_mse_fwd(const void* pred, const void* target, const uint8_t* mask, int64_t N, int64_t C,
